@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — BASELINE.json's metric on the B200 path, and the reference's CPU path beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 Metric: lattice cells x CG iterations per second on the 3D SDF workload (sdf_from_points from a synthetic
 sphere+torus cloud, default Weights), whole job.  A *step* is one pass of the hot path over the cloud:
@@ -74,6 +74,37 @@ def ncu_traffic(workload, precision):
     return t["dram_bytes_per_launch"], f"ncu capture {t.get('captured', '?')} of this kernel build"
 
 
+DUMP_FIELD_VALUES = 1 << 21  # --dump-outputs: field values written over all ranks (8 MB of float32, 24 MB with their indices)
+
+
+def dump_outputs(out_dir, field, stats, rank, world):
+    """--dump-outputs: what the last timed step handed its caller, so that two builds can be compared output for output.
+    field.npy is the solved field (float32) in full when it has at most DUMP_FIELD_VALUES values; a larger one is sampled
+    at indices drawn with a fixed seed and written beside it as field_index.npy (float64, exact for these sizes).  Every
+    solve statistic that is not a time goes to <stat>.npy (float64).  Under torchrun every rank writes its own planes
+    with a _rank<r> suffix.  `field` is a torch tensor (b200 arm) or a numpy array (--impl reference, whose lattice and
+    solver differ from the b200 arm's: its files compare with another run of --impl reference only)."""
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "" if world == 1 else f"_rank{rank}"
+    on_host = isinstance(field, np.ndarray)
+    n, budget = field.size if on_host else field.numel(), DUMP_FIELD_VALUES // world
+    values = field
+    if n > budget:
+        idx = np.sort(np.random.default_rng(0).choice(n, budget, replace=False))
+        np.save(os.path.join(out_dir, f"field_index{suffix}.npy"), idx.astype(np.float64))
+        if on_host:
+            values = field[idx]
+        else:
+            import torch
+            values = field[torch.from_numpy(idx).to(field.device)]
+    if not on_host:
+        values = values.cpu().numpy()
+    np.save(os.path.join(out_dir, f"field{suffix}.npy"), values.astype(np.float32))
+    for name, v in stats.items():
+        if not name.endswith("_ms"):
+            np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), np.array(v, np.float64))
+
+
 class ClockSampler:
     """SM clock and throttle reasons sampled during the timed region (B200_PROFILING.md recipe) through NVML in a
     background thread — the same counters `nvidia-smi --query-gpu=clocks.sm,clocks_event_reasons.*` prints, without
@@ -127,7 +158,8 @@ def cpu_reference_arm(n: int, npts: int, iters: int, budget_s: float, max_steps:
     """The reference's CPU path on this box's host cores: assembly by the reference's own code when oracle/_ref is
     present (else the port), then the restated Eigen path (CSC -> AtA -> Jacobi-preconditioned BiCGSTAB, float) for a
     bounded number of iterations.  Single thread: the reference has no threading.  Runs whole steps (assembly + AtA +
-    `iters` iterations) until `budget_s` is used up, at least one, at most max_steps; returns what actually ran."""
+    `iters` iterations) until `budget_s` is used up, at least one, at most max_steps; returns what actually ran, and the
+    last step's solution and solve stats."""
     from field_interpolation_b200 import workloads as W
     from oracle import oracle as O
     ref = O.reference()
@@ -150,6 +182,7 @@ def cpu_reference_arm(n: int, npts: int, iters: int, budget_s: float, max_steps:
         del N, sys_
         if time.perf_counter() - began + (t3 - t0) > budget_s:
             break
+    last_x, last_stats = x, {"iterations": its, "relative_residual": err}
     total = sum(t for t, _ in times)
     its = sum(i for _, i in times)
     value = (n ** 3) * its / total
@@ -159,7 +192,7 @@ def cpu_reference_arm(n: int, npts: int, iters: int, budget_s: float, max_steps:
         "sample": f"{n}^3 lattice, {npts} points, {len(times)} step(s) of: assembly ({asm_s:.2f} s) + CSC and AtA ({ata_s:.2f} s) + "
                   f"{iters} BiCGSTAB iterations ({it_s:.3f} s each, 2 SpMV per iteration); iterations only: {(n ** 3) / max(it_s, 1e-12):.3e} cell-iters/s",
         "assembly_s": asm_s, "csc_and_ata_s": ata_s, "s_per_bicgstab_iteration": it_s, "steps_run": len(times),
-    }
+    }, last_x, last_stats
 
 
 def cpu_time_to_tol(n: int, npts: int, tol: float = 1e-6):
@@ -369,6 +402,8 @@ def main():
     ap.add_argument("--time-to-tol", action="store_true", help="also time the Jacobi-PCG coarse-to-fine cascade to 1e-6 (slow)")
     ap.add_argument("--no-time-to-tol", action="store_true", help="skip the multigrid time-to-1e-6 measurement")
     ap.add_argument("--mg-timeout", type=float, default=420.0, help="N>1: deadline in seconds for everything after the headline (sharded multigrid time-to-1e-6, slab parity, C5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (solved field, or a seeded sample of it, and its solve stats) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -385,7 +420,9 @@ def main():
         # minutes or in memory it would be honest to ask for; the bounded sample is BASELINE configs[3] (256^3, the same cloud
         # generator) — the b200 arm reports the same configuration in its `configs.C4_sdf3d_256_1M` section.
         sn, snpts, sdesc = WORKLOADS[args.cpu_sample or "sdf3d_256_1M"]
-        value, sec, ran, base = cpu_reference_arm(sn, snpts, args.cpu_iters, args.cpu_budget_s, max(1, args.steps))
+        value, sec, ran, base, last_x, last_stats = cpu_reference_arm(sn, snpts, args.cpu_iters, args.cpu_budget_s, max(1, args.steps))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_x, last_stats, 0, 1)
         base["value"] = value
         base["unit"] = unit
         print(json.dumps({
@@ -444,11 +481,11 @@ def main():
     def step_device():
         if runner is not None:
             st = runner.step(d_pos, d_nrm, opt, d_out)
-            last_stats.update(st)
-            return st
-        f = fi.sdf_from_points(sizes, weights, d_pos, d_nrm)
-        _, st = f.solve(opt, out=d_out)
-        f.close()
+        else:
+            f = fi.sdf_from_points(sizes, weights, d_pos, d_nrm)
+            _, st = f.solve(opt, out=d_out)
+            f.close()
+        last_stats.update(st)
         return st
 
     def step_e2e():
@@ -497,6 +534,8 @@ def main():
     launches = fi.kernel_launches()
     clock_summary = clocks.summary()
     value = N * its / (ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, d_out, last_stats, rank, world)
 
     step_e2e()
     ms_e2e, its_e2e = timed(step_e2e, args.steps)
@@ -652,7 +691,7 @@ def main():
     base = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         sn, snpts, _ = WORKLOADS[args.cpu_sample or "sdf3d_128_1M"]
-        v, sec, _, base = cpu_reference_arm(sn, snpts, 2 * args.cpu_iters, 0.0, 1)
+        v, sec, _, base, _, _ = cpu_reference_arm(sn, snpts, 2 * args.cpu_iters, 0.0, 1)
         base["value"], base["unit"] = v, unit
         # solve against solve, same configuration on both sides: the CPU path to 1e-6 at 64^3 next to the GPU's
         base["time_to_1e-6_64cubed"] = cpu_time_to_tol(64, 100_000)

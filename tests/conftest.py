@@ -75,15 +75,6 @@ def port():
     return O.port()
 
 
-@pytest.fixture(scope="session")
-def ref():
-    from oracle import oracle as O
-    r = O.reference()
-    if r is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    return r
-
-
 @pytest.fixture
 def emu():
     """The package bound to the CPU functional emulator build of the library (tests/emu/) for one test."""

@@ -4,6 +4,15 @@ field_interpolation.cpp compiled unmodified, see oracle/Makefile).  Run in the b
 The fixtures travel to the GPU box (which has no /root/reference); tests compare the CPU port and the
 CUDA path against them.  Solutions are fp64 direct solves (scipy) of the normal equations of the
 reference-assembled rows — the stand-in for solve_sparse_linear_exact (Eigen is not available).
+
+vs_ref.npz holds what the reference returns on the inputs of tests/test_oracle_vs_ref.py.
+
+    python tests/golden/make_golden.py --vs-ref-from-port
+
+writes only vs_ref.npz, from the port instead of the reference.  The committed vs_ref.npz was written that way,
+because the reference's source tree is not part of the repository.  The port, its build flags and the input
+generators are unchanged since commit 4f549c6, where test_oracle_vs_ref ran green against the reference on exactly
+these inputs, and test_oracle_golden still holds the port bit for bit to the fixtures the reference wrote.
 """
 import os
 import sys
@@ -32,7 +41,25 @@ def save(name, sys_, n, **extra):
     print(f"{name}: {sys_.num_rows} rows, {sys_.num_triplets} triplets")
 
 
+def vs_ref(lib):
+    """tests/golden/vs_ref.npz: what `lib` returns on the inputs of tests/test_oracle_vs_ref.py."""
+    sys.path.insert(0, os.path.dirname(OUT))
+    import test_oracle_vs_ref as T
+    out = {}
+    for sizes in T.SDF_SIZES:
+        for vk in (0, 1):
+            for gk in (0, 1, 2):
+                out.update(T.sdf_from_points_outputs(lib, sizes, vk, gk))
+    for make in (T.single_point_builder_outputs, T.upscale_and_error_map_outputs, T.iso_surface_outputs):
+        out.update(make(lib))
+    np.savez_compressed(os.path.join(OUT, "vs_ref"), **T.stored_form(out))
+    print(f"vs_ref: {len(out)} outputs")
+
+
 def main():
+    if "--vs-ref-from-port" in sys.argv:
+        vs_ref(O.port())
+        return
     ref = O.reference()
     assert ref is not None, "build oracle/_ref first (make -C oracle)"
 
@@ -137,6 +164,8 @@ def main():
     iso_case("iso_2x2", np.array([[-1.0, 1.0], [1.0, -2.0]], np.float32), 5, 0.5)
     iso_case("iso_1x7", np.linspace(-1, 1, 7, dtype=np.float32).reshape(1, 7), 2, 0.0)   # no cells at all
     iso_case("iso_9x2", np.linspace(-1, 1, 18, dtype=np.float32).reshape(9, 2), 3, 0.1)
+
+    vs_ref(ref)
 
 
 if __name__ == "__main__":
