@@ -381,6 +381,36 @@ def bicubic_upsample(values, upsample: int):
     return out
 
 
+def marching_cubes(values, iso: float = 0.0, want_normals: bool = False):
+    """Triangle mesh of the surface `values == iso` of a 3D field (fi_marching_cubes, include/fi_b200.h).
+    values: (nz, ny, nx) numpy array or contiguous CUDA tensor, e.g. the `out` of LatticeField.solve.  Returns
+    (vertices (V, 3) float32 in lattice coordinates x y z, triangles (T, 3) int32[, normals (V, 3) float32]), living
+    where `values` lives; triangles are wound so that (P1 - P0) x (P2 - P0) points toward values >= iso."""
+    shape = tuple(values.shape)
+    if len(shape) != 3:
+        raise ValueError("a 3D (nz, ny, nx) field is expected")
+    sizes = (C.c_int32 * 3)(int(shape[2]), int(shape[1]), int(shape[0]))
+    buf = _Buf(values, shape[0] * shape[1] * shape[2])
+    nv, nt = C.c_int64(0), C.c_int64(0)
+    fn = L.lib().fi_marching_cubes
+    L.check(fn(sizes, buf.ptr, float(iso), buf.loc, None, None, 0, None, 0, C.byref(nv), C.byref(nt)))
+    V, T = int(nv.value), int(nt.value)
+    if buf.loc == FI_DEVICE:
+        import torch
+        verts = torch.empty((V, 3), dtype=torch.float32, device=values.device)
+        tris = torch.empty((T, 3), dtype=torch.int32, device=values.device)
+        nrms = torch.empty((V, 3), dtype=torch.float32, device=values.device) if want_normals else None
+        ptr = lambda a: C.c_void_p(a.data_ptr())  # noqa: E731
+    else:
+        verts, tris = np.empty((V, 3), np.float32), np.empty((T, 3), np.int32)
+        nrms = np.empty((V, 3), np.float32) if want_normals else None
+        ptr = lambda a: C.c_void_p(a.ctypes.data)  # noqa: E731
+    if V:
+        L.check(fn(sizes, buf.ptr, float(iso), buf.loc, ptr(verts), ptr(nrms) if want_normals else None, V, ptr(tris), T,
+                   C.byref(nv), C.byref(nt)))
+    return (verts, tris, nrms) if want_normals else (verts, tris)
+
+
 # ---- solvers (sparse_linear.hpp:44-80), on a LatticeField ---------------------------------------------
 # The reference passes field.eq; here the field itself carries the structure (a bare triplet list has lost the
 # lattice).  A failed solve returns an empty array like the reference returns {}.

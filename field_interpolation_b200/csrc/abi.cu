@@ -1067,6 +1067,43 @@ int fi_bicubic_upsample(int32_t width, int32_t height, const float* values, int3
 	});
 }
 
+int fi_marching_cubes(const int32_t* sizes, const float* values, float iso, int32_t loc, float* vertices, float* normals, int64_t capacity_vertices,
+                      int32_t* triangles, int64_t capacity_triangles, int64_t* num_vertices, int64_t* num_triangles)
+{
+	return guarded([&] {
+		FI_REQUIRE(sizes && values && num_vertices && num_triangles, FI_ERR_INVALID, "marching cubes: null argument");
+		FI_REQUIRE(sizes[0] >= 1 && sizes[1] >= 1 && sizes[2] >= 1, FI_ERR_INVALID, "marching cubes: size < 1");
+		FI_REQUIRE(((vertices || normals) ? capacity_vertices >= 0 : true) && (triangles ? capacity_triangles >= 0 : true), FI_ERR_INVALID,
+		           "marching cubes: negative capacity");
+		*num_vertices  = 0;
+		*num_triangles = 0;
+		const int64_t nnodes = static_cast<int64_t>(sizes[0]) * sizes[1] * sizes[2];
+		FI_REQUIRE(nnodes < (int64_t{1} << 31), FI_ERR_RANGE, "marching cubes: more than 2^31 - 1 nodes");
+		cudaStream_t  s = nullptr;
+		Staged<float> v(values, static_cast<size_t>(nnodes), loc, s);
+		const bool    fill = vertices || normals || triangles;
+		McCounts      n;
+		if (loc == FI_DEVICE || !fill) {
+			n = marching_cubes_device(sizes, v.ptr, iso, vertices, normals, capacity_vertices, triangles, capacity_triangles, s);
+		} else {
+			n = marching_cubes_device(sizes, v.ptr, iso, nullptr, nullptr, 0, nullptr, 0, s);
+		}
+		*num_vertices  = n.vertices;
+		*num_triangles = n.triangles;
+		FI_REQUIRE(!(vertices || normals) || n.vertices <= capacity_vertices, FI_ERR_RANGE, "marching cubes: vertex buffer too small");
+		FI_REQUIRE(!triangles || n.triangles <= capacity_triangles, FI_ERR_RANGE, "marching cubes: triangle buffer too small");
+		if (loc == FI_DEVICE || !fill || n.vertices == 0) { return; }
+		const size_t  nv = static_cast<size_t>(n.vertices) * 3, nt = static_cast<size_t>(n.triangles) * 3;
+		DevBuf<float> dv(vertices ? nv : 0), dn(normals ? nv : 0);
+		DevBuf<int32_t> dt(triangles ? nt : 0);
+		marching_cubes_device(sizes, v.ptr, iso, vertices ? dv.data() : nullptr, normals ? dn.data() : nullptr, n.vertices,
+		                      triangles ? dt.data() : nullptr, n.triangles, s);
+		if (vertices) { FI_CUDA(cudaMemcpy(vertices, dv.data(), nv * sizeof(float), cudaMemcpyDeviceToHost)); }
+		if (normals) { FI_CUDA(cudaMemcpy(normals, dn.data(), nv * sizeof(float), cudaMemcpyDeviceToHost)); }
+		if (triangles) { FI_CUDA(cudaMemcpy(triangles, dt.data(), nt * sizeof(int32_t), cudaMemcpyDeviceToHost)); }
+	});
+}
+
 int fi_sdf_solve_cascade(int32_t ndim, const int32_t* sizes, const fi_weights* w, int64_t num_points, const float* unit_positions,
                          const float* normals, const float* point_weights, const fi_cascade_options* opt, float* solution,
                          int32_t loc, fi_cascade_stats* stats)

@@ -180,6 +180,18 @@ int64_t marching_squares_device(int width, int height, const float* d_values, fl
 double  area_twice_device(int64_t nseg, const float* d_lines, cudaStream_t s);
 void    bicubic_upsample_device(int width, int height, const float* d_values, int upsample, float* d_large, cudaStream_t s);
 
+// ---- marching_cubes.cuh (included by isosurface.cu, compiled with -fmad=false) --------------------------------------
+// Mesh of `values == iso` of a sizes[0] x sizes[1] x sizes[2] lattice (x fastest) on the device; the contract is in
+// include/fi_b200.h (fi_marching_cubes).  Always returns the counts.  Vertices / normals (3 floats each, nullable) and
+// triangles (3 int32 each, nullable) are written only when every requested buffer holds its count; all outputs
+// nullptr: count only.
+struct McCounts
+{
+	int64_t vertices = 0, triangles = 0;
+};
+McCounts marching_cubes_device(const int32_t* sizes, const float* d_values, float iso, float* d_vertices, float* d_normals,
+                               int64_t capacity_vertices, int32_t* d_triangles, int64_t capacity_triangles, cudaStream_t s);
+
 // ---- stencil.cu ------------------------------------------------------------------------------------------
 // Per-axis banded operator T_d = sum_k w_k^2 D_k^T D_k (rows that stick out dropped), 9 row classes x 9 taps,
 // plus the tri-diagonal D_1^T D_1 used by the gradient-smoothness cross terms.  See DESIGN.md §3.

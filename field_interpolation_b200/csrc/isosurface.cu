@@ -249,3 +249,6 @@ void bicubic_upsample_device(int width, int height, const float* d_values, int u
 }
 
 }  // namespace fi
+
+// The 3D counterpart, marching cubes, shares this translation unit and its -fmad=false build.
+#include "marching_cubes.cuh"

@@ -1,9 +1,12 @@
-// Host side of include/emilib/marching_squares.hpp and include/field_interpolation/iso_surface.hpp: thin C++ over the
-// C ABI (fi_marching_squares, fi_calc_area, fi_bicubic_upsample).  No arithmetic happens here.
+// Host side of include/emilib/marching_squares.hpp, include/field_interpolation/iso_surface.hpp and
+// b200::marching_cubes: thin C++ over the C ABI (fi_marching_squares, fi_calc_area, fi_bicubic_upsample,
+// fi_marching_cubes).  No arithmetic happens here.
 #include "../../include/emilib/marching_squares.hpp"
+#include "../../include/field_interpolation/field_interpolation.hpp"
 #include "../../include/field_interpolation/iso_surface.hpp"
 
 #include <cstdint>
+#include <utility>
 
 #include "../../include/fi_b200.h"
 
@@ -52,4 +55,32 @@ std::vector<float> bicubic_upsample(int* io_width, int* io_height, const float* 
 
 std::vector<float> iso_surface(int width, int height, const float* values, float iso) { return contour(width, height, values, iso); }
 
+}  // namespace field_interpolation
+
+namespace field_interpolation {
+namespace b200 {
+
+bool marching_cubes(const std::vector<int>& sizes, const float* values, float iso, bool want_normals, Mesh* mesh)
+{
+	if (mesh == nullptr) { return false; }
+	*mesh = Mesh();
+	if (sizes.size() != 3 || values == nullptr) { return false; }
+	const int32_t sz[3] = {sizes[0], sizes[1], sizes[2]};
+	int64_t       nv = 0, nt = 0;
+	if (fi_marching_cubes(sz, values, iso, FI_HOST, nullptr, nullptr, 0, nullptr, 0, &nv, &nt) != FI_OK) { return false; }
+	if (nv == 0) { return true; }
+	Mesh out;
+	out.positions.resize(static_cast<size_t>(nv) * 3);
+	if (want_normals) { out.normals.resize(static_cast<size_t>(nv) * 3); }
+	out.triangles.resize(static_cast<size_t>(nt) * 3);
+	static_assert(sizeof(int) == sizeof(int32_t), "triangles are int32 in the C ABI");
+	if (fi_marching_cubes(sz, values, iso, FI_HOST, out.positions.data(), want_normals ? out.normals.data() : nullptr, nv,
+	                      reinterpret_cast<int32_t*>(out.triangles.data()), nt, &nv, &nt) != FI_OK) {
+		return false;
+	}
+	*mesh = std::move(out);
+	return true;
+}
+
+}  // namespace b200
 }  // namespace field_interpolation

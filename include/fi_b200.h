@@ -26,7 +26,8 @@ extern "C" {
 #endif
 
 /* 2: + fi_marching_squares, fi_calc_area, fi_bicubic_upsample, fi_slab_balanced_cuts, fi_comm_set_slab_cuts (additions only) */
-#define FI_B200_ABI_VERSION 3
+/* 4: + fi_marching_cubes (additions only) */
+#define FI_B200_ABI_VERSION 4
 
 #if defined(__GNUC__)
 #define FI_API __attribute__((visibility("default")))
@@ -224,6 +225,24 @@ FI_API int fi_calc_area(int64_t num_segments, const float* lines, int32_t loc, f
  * (upsample * width - upsample + 1) x (upsample * height - upsample + 1), clamped reads at the border; upsample >= 2
  * (the reference CHECKs > 1).  Bit-identical fp32 arithmetic. */
 FI_API int fi_bicubic_upsample(int32_t width, int32_t height, const float* values, int32_t upsample, float* large, int32_t loc);
+/* Triangle mesh of the surface values == iso of a 3D lattice (x fastest), in lattice coordinates.
+ * sizes: nx, ny, nz.  A node is outside when value - iso >= 0 (-0.0 and exact zeros included), as in marching squares.
+ * Vertices: one per lattice edge whose two end nodes lie on different sides, numbered by (lower end node's linear index,
+ * then axis x < y < z); the coordinate along the edge is float(coord_lo) + a / (a - b) with a, b = the lower and upper
+ * end's value - iso, the other two are the node's.  Normals (optional): the central-difference gradient of the values
+ * (one-sided at the border) at both ends, interpolated with t = a / (a - b) and normalised (zero stays zero); they
+ * point toward increasing values.  Triangles: three int32 vertex indices each, in cell order (cell = its lowest node)
+ * and case-table order within a cell, wound so that (P1 - P0) x (P2 - P0) points to the outside side.  Each cell
+ * face is resolved from its own four corners the way fi_marching_squares resolves a saddle, so the mesh is crack-free
+ * and its cross-section on every lattice face is that plane's marching-squares contour.  Deterministic.
+ * *num_vertices and *num_triangles always receive the counts.  vertices / normals (3 floats per vertex) and triangles
+ * are nullable (all null: count only); when a count exceeds its capacity nothing is written and the call returns
+ * FI_ERR_RANGE.  values and all outputs live where `loc` says (device outputs need 4-byte alignment only).  Any size
+ * < 2 gives an empty mesh; more than 2^31 - 1 nodes or vertices: FI_ERR_RANGE. */
+FI_API int fi_marching_cubes(const int32_t* sizes /* 3 */, const float* values, float iso, int32_t loc,
+                             float* vertices /* 3 per vertex, nullable */, float* normals /* 3 per vertex, nullable */,
+                             int64_t capacity_vertices, int32_t* triangles /* 3 per triangle, nullable */,
+                             int64_t capacity_triangles, int64_t* num_vertices, int64_t* num_triangles);
 
 /* Coarse-to-fine solve mirroring the demo's recipe (src/sdf_field.cpp:251-304) applied recursively:
  * positions are in UNIT coordinates and are scaled per level by (size-1) as on_lattice does (:198-210);

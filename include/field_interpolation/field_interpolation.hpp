@@ -126,6 +126,17 @@ std::vector<float> sdf_solve_cascade(const std::vector<int>& sizes, const Weight
                                      const float* normals, const float* point_weights, Precision precision, int max_iterations,
                                      double tolerance, int factor, int coarsest_size, double coarse_tolerance, CascadeStats* stats);
 
+/// Triangle mesh in lattice coordinates (x y z per vertex; three vertex indices per triangle).
+struct Mesh
+{
+	std::vector<float> positions, normals;  ///< 3 floats per vertex; normals empty unless asked for
+	std::vector<int>   triangles;           ///< 3 per triangle, (P1 - P0) x (P2 - P0) toward values >= iso
+};
+
+/// Marching cubes of the surface values == iso of a 3D lattice (sizes = {nx, ny, nz}, x fastest, host values) on the
+/// GPU: fi_marching_cubes (include/fi_b200.h) states the contract.  Returns false on failure (mesh left empty).
+bool marching_cubes(const std::vector<int>& sizes, const float* values, float iso, bool want_normals, Mesh* mesh);
+
 }  // namespace b200
 
 }  // namespace field_interpolation
