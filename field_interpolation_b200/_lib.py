@@ -99,6 +99,7 @@ SIGNATURES = {
     "fi_calc_area": (C.c_int, [_i64, _vp, _i32, _pf]),
     "fi_bicubic_upsample": (C.c_int, [_i32, _i32, _vp, _i32, _vp, _i32]),
     "fi_marching_cubes": (C.c_int, [_pi32, _vp, _f, _i32, _vp, _vp, _i64, _vp, _i64, _pi64, _pi64]),
+    "fi_sample_field": (C.c_int, [_i32, _pi32, _vp, _i64, _vp, _i32, _i32, _vp, _vp]),
     "fi_sdf_solve_cascade": (C.c_int, [_i32, _pi32, _p(fi_weights), _i64, _vp, _vp, _vp, _p(fi_cascade_options), _vp, _i32,
                                        _p(fi_cascade_stats)]),
     "fi_comm_unique_id": (C.c_int, [_vp, _i64]),

@@ -411,6 +411,43 @@ def marching_cubes(values, iso: float = 0.0, want_normals: bool = False):
     return (verts, tris, nrms) if want_normals else (verts, tris)
 
 
+def sample_field(field, positions, gradient_kernel=None):
+    """Value (and gradient) of a lattice field at arbitrary points (fi_sample_field, include/fi_b200.h).
+    field: (n,), (ny, nx) or (nz, ny, nx), numpy array or CUDA tensor; positions: (N, D) lattice coordinates, columns
+    x y z, living where `field` lives.  gradient_kernel: None (values only) or a GradientKernel.  Returns values (N,)
+    float32, or (values, gradients (N, D)) when a kernel is given, living where the inputs live.  Points where the
+    reference would emit no row (outside the lattice, non-finite) read NaN."""
+    shape = tuple(field.shape)
+    D = len(shape)
+    if D not in (1, 2, 3):
+        raise ValueError("a (n,), (ny, nx) or (nz, ny, nx) field is expected")
+    pshape = tuple(positions.shape)
+    if len(pshape) != 2 or pshape[1] != D:
+        raise ValueError(f"positions must be (N, {D})")
+    if _is_device(field) != _is_device(positions):
+        raise ValueError("field and positions must live in the same place (both host or both device)")
+    if _is_device(field):
+        field, positions = field.contiguous(), positions.contiguous()
+    N = int(pshape[0])
+    sizes = (C.c_int32 * D)(*[int(s) for s in reversed(shape)])
+    fb = _Buf(field, int(np.prod(shape, dtype=np.int64)))
+    pb = _Buf(positions, N * D)
+    want = gradient_kernel is not None
+    if fb.loc == FI_DEVICE:
+        import torch
+        vals = torch.empty(N, dtype=torch.float32, device=field.device)
+        grads = torch.empty((N, D), dtype=torch.float32, device=field.device) if want else None
+        ptr = lambda a: C.c_void_p(a.data_ptr())  # noqa: E731
+    else:
+        vals = np.empty(N, np.float32)
+        grads = np.empty((N, D), np.float32) if want else None
+        ptr = lambda a: C.c_void_p(a.ctypes.data)  # noqa: E731
+    if N:
+        L.check(L.lib().fi_sample_field(D, sizes, fb.ptr, N, pb.ptr, int(gradient_kernel) if want else 0, fb.loc, ptr(vals),
+                                        ptr(grads) if want else None))
+    return (vals, grads) if want else vals
+
+
 # ---- solvers (sparse_linear.hpp:44-80), on a LatticeField ---------------------------------------------
 # The reference passes field.eq; here the field itself carries the structure (a bare triplet list has lost the
 # lattice).  A failed solve returns an empty array like the reference returns {}.

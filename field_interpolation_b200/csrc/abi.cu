@@ -1104,6 +1104,36 @@ int fi_marching_cubes(const int32_t* sizes, const float* values, float iso, int3
 	});
 }
 
+int fi_sample_field(int32_t ndim, const int32_t* sizes, const float* field, int64_t num_points, const float* positions,
+                    int32_t gradient_kernel, int32_t loc, float* values, float* gradients)
+{
+	return guarded([&] {
+		FI_REQUIRE(1 <= ndim && ndim <= kMaxDim, FI_ERR_INVALID, "sample_field: ndim must be 1..3");
+		FI_REQUIRE(loc == FI_HOST || loc == FI_DEVICE, FI_ERR_INVALID, "sample_field: unknown loc");
+		FI_REQUIRE(num_points >= 0, FI_ERR_INVALID, "sample_field: negative num_points");
+		FI_REQUIRE(!gradients || (0 <= gradient_kernel && gradient_kernel <= 2), FI_ERR_INVALID, "sample_field: unknown gradient kernel");
+		if (sizes) {
+			for (int d = 0; d < ndim; ++d) { FI_REQUIRE(sizes[d] >= 1, FI_ERR_INVALID, "sample_field: size must be >= 1"); }
+		}
+		if (num_points == 0) { return; }
+		FI_REQUIRE(sizes && field && positions, FI_ERR_INVALID, "sample_field: null argument");
+		if (!values && !gradients) { return; }
+		const Geom    g = make_geom(ndim, sizes);
+		const size_t  np = static_cast<size_t>(num_points), nd = np * static_cast<size_t>(ndim);
+		cudaStream_t  s = nullptr;
+		Staged<float> x(field, static_cast<size_t>(g.N), loc, s), p(positions, nd, loc, s);
+		if (loc == FI_DEVICE) {
+			sample_field_device(g, num_points, p.ptr, x.ptr, gradient_kernel, values, gradients, s);
+			FI_CUDA(cudaStreamSynchronize(s));
+			return;
+		}
+		DevBuf<float> v(values ? np : 0), gr(gradients ? nd : 0);
+		sample_field_device(g, num_points, p.ptr, x.ptr, gradient_kernel, values ? v.data() : nullptr, gradients ? gr.data() : nullptr, s);
+		if (values) { FI_CUDA(cudaMemcpy(values, v.data(), np * sizeof(float), cudaMemcpyDeviceToHost)); }
+		if (gradients) { FI_CUDA(cudaMemcpy(gradients, gr.data(), nd * sizeof(float), cudaMemcpyDeviceToHost)); }
+	});
+}
+
 int fi_sdf_solve_cascade(int32_t ndim, const int32_t* sizes, const fi_weights* w, int64_t num_points, const float* unit_positions,
                          const float* normals, const float* point_weights, const fi_cascade_options* opt, float* solution,
                          int32_t loc, fi_cascade_stats* stats)

@@ -1368,3 +1368,6 @@ template bool apply_data_term<float>(const Geom&, const DataTerm<float>&, const 
 template bool apply_data_term<double>(const Geom&, const DataTerm<double>&, const double*, double*, double*, const int*, cudaStream_t, const PeerPublish*);
 
 }  // namespace fi
+
+// Point sampling (value and gradient at arbitrary positions) shares this translation unit and its -fmad=false build.
+#include "sample_field.cuh"

@@ -117,6 +117,11 @@ void emit_model_rows(const Geom& g, const fi_weights& w, const uint64_t* d_rowof
                      int64_t row_base, int64_t trip_base, fi_triplet* d_trips, float* d_rhs, cudaStream_t s);
 void upscale_device(const Geom& small, const Geom& large, const float* d_small, float* d_large, float post_scale,
                     cudaStream_t s);
+// sample_field.cuh (included by assembly.cu): value (d_values, nullable) and gradient (d_gradients, D per point,
+// nullable; gradient_kernel 0..2) of the unsharded lattice field at n interleaved positions; fi_sample_field states
+// the contract.
+void sample_field_device(const Geom& g, int64_t n, const float* d_positions, const float* d_field, int gradient_kernel,
+                         float* d_values, float* d_gradients, cudaStream_t s);
 
 // Data term of the normal equations in compact form: per occupied cell a symmetric 2^D x 2^D block
 // (upper triangle, struct-of-arrays [tri][cell]) plus the rows that do not fit a cell (linear-interpolation

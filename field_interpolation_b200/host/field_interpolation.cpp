@@ -4,6 +4,7 @@
 // kernels of csrc/assembly.cu.
 #include <cmath>
 #include <cstring>
+#include <utility>
 
 #include "structured.hpp"
 
@@ -239,6 +240,24 @@ std::vector<float> sdf_solve_cascade(const std::vector<int>& sizes, const Weight
 		stats->finest.generic_rows      = cs.finest.generic_rows;
 	}
 	return out;
+}
+
+bool sample_field(const std::vector<int>& sizes, const float* field, int64_t num_points, const float* positions, GradientKernel kernel,
+                  bool want_gradients, std::vector<float>* values, std::vector<float>* gradients)
+{
+	if (values) { values->clear(); }
+	if (gradients) { gradients->clear(); }
+	if (values == nullptr || (want_gradients && gradients == nullptr) || sizes.empty() || sizes.size() > 3 || num_points < 0) { return false; }
+	const int32_t              ndim = static_cast<int32_t>(sizes.size());
+	const std::vector<int32_t> sz(sizes.begin(), sizes.end());
+	std::vector<float>         v(static_cast<size_t>(num_points)), g(want_gradients ? static_cast<size_t>(num_points) * ndim : 0);
+	if (fi_sample_field(ndim, sz.data(), field, num_points, positions, static_cast<int32_t>(kernel), FI_HOST, v.data(),
+	                    want_gradients ? g.data() : nullptr) != FI_OK) {
+		return false;
+	}
+	*values = std::move(v);
+	if (want_gradients) { *gradients = std::move(g); }
+	return true;
 }
 
 }  // namespace b200

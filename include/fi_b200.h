@@ -27,7 +27,8 @@ extern "C" {
 
 /* 2: + fi_marching_squares, fi_calc_area, fi_bicubic_upsample, fi_slab_balanced_cuts, fi_comm_set_slab_cuts (additions only) */
 /* 4: + fi_marching_cubes (additions only) */
-#define FI_B200_ABI_VERSION 4
+/* 5: + fi_sample_field (additions only) */
+#define FI_B200_ABI_VERSION 5
 
 #if defined(__GNUC__)
 #define FI_API __attribute__((visibility("default")))
@@ -243,6 +244,33 @@ FI_API int fi_marching_cubes(const int32_t* sizes /* 3 */, const float* values, 
                              float* vertices /* 3 per vertex, nullable */, float* normals /* 3 per vertex, nullable */,
                              int64_t capacity_vertices, int32_t* triangles /* 3 per triangle, nullable */,
                              int64_t capacity_triangles, int64_t* num_vertices, int64_t* num_triangles);
+/* Value and, optionally, gradient of a lattice field (x fastest) at arbitrary points, as the reference's constraint
+ * rows measure them (field_interpolation.cpp:57-80, :123-240).  positions: D interleaved floats per point in lattice
+ * coordinates, as fi_field_add_points takes them.  Outputs are in caller order, each the fp32 expression below with no
+ * FMA contraction:
+ *   value      upscale_field's expression (:431-485) at p: over the in-lattice corners of cell floor(p), in ascending
+ *              corner order, wsum = sum k and fsum = sum k * x sequentially, then fsum / wsum.  This is what a
+ *              linear-interpolation value row sees (coefficients k * w, rhs w * sum k * value); it is defined on
+ *              (-1, n_d) per axis, partly outside cells use the normalised partial sum, and where wsum == 0 (no row)
+ *              the value is NaN, not the 0 that fi_upscale_field writes.
+ *   gradient   (gradients != null) what an add_gradient_constraint(p, ., weight 1, gradient_kernel) row measures:
+ *              FI_GRADIENT_NEAREST_NEIGHBOR      x[cell + s_d] - x[cell], cell = floor(p);
+ *              FI_GRADIENT_CELL_EDGES            acc = acc + (+-2 / 2^D) * x[corner] over the cell's corners in
+ *                                                order, + where corner bit d is set;
+ *              FI_GRADIENT_LINEAR_INTERPOLATION  the corners of floor(p - 0.5) with c + 1 < n_d, weights k:
+ *                                                acc = acc + (-k) * x[i], acc = acc + k * x[i + s_d] per corner in
+ *                                                order, then acc / sum k.
+ *              NaN in every component where the reference emits no row: kernels 0 and 1 when the cell is not
+ *              entirely inside, kernel 2 when no corner is kept or the kept weights sum to 0.
+ * NaN or infinite positions, and positions outside the lattice (however far), give NaN outputs.  The
+ * nearest-neighbour value kernel (:82-107) is not offered: its prediction depends on each point's normal.
+ * field, positions, values (nullable) and gradients (D per point, nullable) live where `loc` says; device buffers need
+ * 4-byte alignment only.  num_points == 0 is a no-op.  FI_ERR_INVALID: ndim outside 1..3, a size < 1, an unknown loc,
+ * a negative count, null sizes / field / positions with points present, an unknown gradient_kernel with gradients
+ * != null. */
+FI_API int fi_sample_field(int32_t ndim, const int32_t* sizes, const float* field, int64_t num_points,
+                           const float* positions /* D per point, lattice coordinates */, int32_t gradient_kernel,
+                           int32_t loc, float* values /* nullable */, float* gradients /* D per point, nullable */);
 
 /* Coarse-to-fine solve mirroring the demo's recipe (src/sdf_field.cpp:251-304) applied recursively:
  * positions are in UNIT coordinates and are scaled per level by (size-1) as on_lattice does (:198-210);

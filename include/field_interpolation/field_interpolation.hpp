@@ -11,6 +11,7 @@
 // triplet list stays observable and appendable exactly as before.
 #pragma once
 
+#include <cstdint>
 #include <vector>
 
 #include "sparse_linear.hpp"
@@ -136,6 +137,13 @@ struct Mesh
 /// Marching cubes of the surface values == iso of a 3D lattice (sizes = {nx, ny, nz}, x fastest, host values) on the
 /// GPU: fi_marching_cubes (include/fi_b200.h) states the contract.  Returns false on failure (mesh left empty).
 bool marching_cubes(const std::vector<int>& sizes, const float* values, float iso, bool want_normals, Mesh* mesh);
+
+/// Value (and gradient) of a lattice field (sizes = {nx[, ny[, nz]]}, x fastest, host values) at num_points host
+/// positions (D interleaved floats each, lattice coordinates), on the GPU: fi_sample_field (include/fi_b200.h) states
+/// the contract.  values receives num_points floats; gradients (with want_gradients) D per point, computed with
+/// `kernel`.  NaN where the reference would emit no row.  Returns false on failure (outputs left empty).
+bool sample_field(const std::vector<int>& sizes, const float* field, int64_t num_points, const float* positions, GradientKernel kernel,
+                  bool want_gradients, std::vector<float>* values, std::vector<float>* gradients);
 
 }  // namespace b200
 
