@@ -95,6 +95,7 @@ SIGNATURES = {
     "fi_field_jacobi": (C.c_int, [_vp, _pf, _i32, _f, _pf]),
     "fi_upscale_field": (C.c_int, [_i32, _pi32, _pi32, _vp, _vp, _i32]),
     "fi_error_map": (C.c_int, [_i64, _vp, _i64, _pf, _i64, _pf, _pf]),
+    "fi_field_error_map": (C.c_int, [_vp, _vp, _i32, _vp, _pd]),
     "fi_marching_squares": (C.c_int, [_i32, _i32, _vp, _f, _i32, _vp, _i64, _pi64, _pf]),
     "fi_calc_area": (C.c_int, [_i64, _vp, _i32, _pf]),
     "fi_bicubic_upsample": (C.c_int, [_i32, _i32, _vp, _i32, _vp, _i32]),

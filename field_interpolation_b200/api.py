@@ -448,6 +448,28 @@ def sample_field(field, positions, gradient_kernel=None):
     return (vals, grads) if want else vals
 
 
+def generate_error_map(field: LatticeField, solution, want_sums: bool = False):
+    """generate_error_map (field_interpolation.cpp:402-429) of the field's own system (fi_field_error_map,
+    include/fi_b200.h): bit-identical to the reference's function on field.eq, computed on the device without the
+    triplet list.  Like the solvers, it takes the field where the reference takes field.eq.  solution: N floats,
+    numpy array or CUDA tensor.  Returns the heat map (N,) float32, living where `solution` lives; with want_sums
+    also the fp64 sums of err^2 over model, point and caller rows (a (3,) float64 numpy array)."""
+    if _is_device(solution):
+        solution = solution.contiguous()
+    N = field.num_unknowns
+    sol = _Buf(solution, N)
+    if sol.loc == FI_DEVICE:
+        import torch
+        heat = torch.empty(N, dtype=torch.float32, device=solution.device)
+        dst = C.c_void_p(heat.data_ptr())
+    else:
+        heat = np.empty(N, np.float32)
+        dst = C.c_void_p(heat.ctypes.data)
+    sums = (C.c_double * 3)()
+    L.check(L.lib().fi_field_error_map(field._h, sol.ptr, sol.loc, dst, sums))
+    return (heat, np.array(sums[:], np.float64)) if want_sums else heat
+
+
 # ---- solvers (sparse_linear.hpp:44-80), on a LatticeField ---------------------------------------------
 # The reference passes field.eq; here the field itself carries the structure (a bare triplet list has lost the
 # lattice).  A failed solve returns an empty array like the reference returns {}.

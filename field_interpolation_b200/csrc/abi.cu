@@ -1011,6 +1011,47 @@ int fi_error_map(int64_t num_triplets, const fi_triplet* triplets, int64_t num_c
 	});
 }
 
+int fi_field_error_map(fi_field* f, const float* solution, int32_t loc, float* heatmap, double* row_error_sums)
+{
+	return guarded([&] {
+		TraceScope trace("fi_field_error_map");
+		FI_REQUIRE(f && solution && heatmap, FI_ERR_INVALID, "field_error_map: null argument");
+		FI_REQUIRE(loc == FI_HOST || loc == FI_DEVICE, FI_ERR_INVALID, "field_error_map: unknown loc");
+		bool emitted_rows = false;  // point and caller rows go through int32 columns (the emitters' triplets)
+		for (const Segment& sg : f->segs) {
+			emitted_rows = emitted_rows || (sg.kind == Segment::kPoints && sg.p1 > sg.p0) || (sg.kind == Segment::kRows && sg.r1 > sg.r0);
+		}
+		FI_REQUIRE(!emitted_rows || f->g.N <= INT32_MAX, FI_ERR_RANGE, "field_error_map: point or caller rows on more than 2^31 - 1 nodes");
+		const int64_t N = f->g.N;
+		cudaStream_t  s = f->stream;
+		Staged<float> x(solution, static_cast<size_t>(N), loc, s);
+		DevBuf<float> own;
+		float*        heat = heatmap;
+		if (loc != FI_DEVICE) {
+			own.resize(N);
+			heat = own.data();
+		}
+		FI_CUDA(cudaMemsetAsync(heat, 0, N * sizeof(float), s));
+		DevBuf<double> sums(3);
+		sums.zero(s);
+		ErrorMapScratch sc;
+		for (const Segment& sg : f->segs) {  // in builder-call order: every column receives its terms in global triplet order
+			if (sg.kind == Segment::kModel) {
+				model_error_map(f->g, sg.w, x.ptr, heat, sums.data() + 0, sc, s);
+			} else if (sg.kind == Segment::kPoints) {
+				point_error_map(f->g, view(f->pts), sg.p0, sg.p1, x.ptr, heat, sums.data() + 1, sc, s);
+			} else {
+				caller_rows_error_map(f->g, f->rows, sg.r0, sg.r1, x.ptr, heat, sums.data() + 2, sc, s);
+			}
+		}
+		double h[3];
+		FI_CUDA(cudaMemcpyAsync(h, sums.data(), sizeof(h), cudaMemcpyDeviceToHost, s));
+		if (loc != FI_DEVICE) { FI_CUDA(cudaMemcpyAsync(heatmap, heat, N * sizeof(float), cudaMemcpyDeviceToHost, s)); }
+		FI_CUDA(cudaStreamSynchronize(s));
+		if (row_error_sums) { std::memcpy(row_error_sums, h, sizeof(h)); }
+	});
+}
+
 int fi_marching_squares(int32_t width, int32_t height, const float* values, float iso, int32_t loc, float* lines, int64_t capacity_segments,
                         int64_t* num_segments, float* area)
 {

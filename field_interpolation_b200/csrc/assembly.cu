@@ -1371,3 +1371,5 @@ template bool apply_data_term<double>(const Geom&, const DataTerm<double>&, cons
 
 // Point sampling (value and gradient at arbitrary positions) shares this translation unit and its -fmad=false build.
 #include "sample_field.cuh"
+// So does the error map of a field's own system (bit-identical to generate_error_map on its exported triplets).
+#include "field_error_map.cuh"

@@ -177,6 +177,27 @@ template <typename T>
 bool apply_data_term_epilogue(const Geom& g, const DataTerm<T>& dt, const T* in, T* res_out, const T* minv, T* e, T* d_new, T b,
                               cudaStream_t s);
 
+// ---- field_error_map.cuh (included by assembly.cu, compiled with -fmad=false) ---------------------------------
+// generate_error_map of the rows one builder call added, from the field's own description; fi_field_error_map states
+// the contract.  Each adds the segment's terms to d_heat (device, N floats) in the segment's triplet order and the
+// fp64 sum of its rows' err^2 to *d_sum (device).  Point and caller rows go through scratch of at most
+// error_map_chunk_triplets() triplets at a time (2^26; FI_B200_ERROR_MAP_CHUNK overrides it).
+struct ErrorMapScratch
+{
+	DevBuf<uint64_t>   rowoff, tripoff, row_ptr, key;
+	DevBuf<uint32_t>   idx;
+	DevBuf<fi_triplet> trips;
+	DevBuf<int32_t>    col;
+	DevBuf<float>      val, rhs, term;
+	DevBuf<double>     partial;
+};
+int64_t error_map_chunk_triplets();
+void    model_error_map(const Geom& g, const fi_weights& w, const float* d_x, float* d_heat, double* d_sum, ErrorMapScratch& sc, cudaStream_t s);
+void    point_error_map(const Geom& g, PointView pv, int64_t p0, int64_t p1, const float* d_x, float* d_heat, double* d_sum, ErrorMapScratch& sc,
+                        cudaStream_t s);
+void    caller_rows_error_map(const Geom& g, const HostRows& rows, int64_t r0, int64_t r1, const float* d_x, float* d_heat, double* d_sum,
+                              ErrorMapScratch& sc, cudaStream_t s);
+
 // ---- errormap.cu ------------------------------------------------------------------------------------------
 void error_map(int64_t nt, const fi_triplet* h_trips, int64_t n, const float* h_x, int64_t nrows, const float* h_rhs, float* h_out);
 

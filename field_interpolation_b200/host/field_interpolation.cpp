@@ -260,6 +260,25 @@ bool sample_field(const std::vector<int>& sizes, const float* field, int64_t num
 	return true;
 }
 
+std::vector<float> generate_error_map(LatticeField* field, const std::vector<float>& solution, ErrorSums* sums)
+{
+	if (field == nullptr) { return {}; }
+	Structured* st = structured_for_append(field);  // forwards rows appended to field->eq by hand since the last builder call
+	if (!st) { return {}; }
+	size_t n = 1;
+	for (int s : field->sizes) { n *= static_cast<size_t>(s); }
+	if (solution.size() != n) { return {}; }
+	std::vector<float> heat(n);
+	double             s[3] = {0, 0, 0};
+	if (fi_field_error_map(st->handle, solution.data(), FI_HOST, heat.data(), s) != FI_OK) { return {}; }
+	if (sums) {
+		sums->model_rows  = s[0];
+		sums->point_rows  = s[1];
+		sums->caller_rows = s[2];
+	}
+	return heat;
+}
+
 }  // namespace b200
 
 using b200::build;

@@ -28,7 +28,8 @@ extern "C" {
 /* 2: + fi_marching_squares, fi_calc_area, fi_bicubic_upsample, fi_slab_balanced_cuts, fi_comm_set_slab_cuts (additions only) */
 /* 4: + fi_marching_cubes (additions only) */
 /* 5: + fi_sample_field (additions only) */
-#define FI_B200_ABI_VERSION 5
+/* 6: + fi_field_error_map (additions only) */
+#define FI_B200_ABI_VERSION 6
 
 #if defined(__GNUC__)
 #define FI_API __attribute__((visibility("default")))
@@ -209,6 +210,22 @@ FI_API int fi_upscale_field(int32_t ndim, const int32_t* small_sizes, const int3
  * by squared coefficient.  Any triplet list (rows need not be grouped).  Host buffers; heatmap: num_columns floats. */
 FI_API int fi_error_map(int64_t num_triplets, const fi_triplet* triplets, int64_t num_columns, const float* solution,
                  int64_t num_rows, const float* rhs, float* heatmap);
+
+/* generate_error_map of the field's own system, computed on the device from what the field holds (no triplet list,
+ * no O(rows) host buffer; deferred fields and systems beyond fi_field_export's int32 limits included).
+ * heatmap (N floats) is bit-identical to generate_error_map (field_interpolation.cpp:402-429) applied to the triplets
+ * and rhs fi_field_export would write for f, for every mix and order of builder calls and for clones:
+ *   per row, err = rhs; err -= x[col] * v and sq += v * v in triplet order; then err *= err;
+ *   then out[col] += (v * v) / sq * err in global triplet order, skipped where sq == 0
+ * (fp32, no FMA contraction; NaN in the solution propagates as that arithmetic propagates it).
+ * row_error_sums (nullable, 3 doubles) receives sum over rows of err^2 — err the fp32 row error above, squared and
+ * summed in fp64 — split into [0] model rows, [1] point rows, [2] caller rows: the least-squares objective the solve
+ * minimises, by term.  The sums are reduced in a fixed order and repeat bit for bit from run to run.
+ * solution and heatmap live where `loc` says; device buffers need 4-byte alignment only.  A field without rows gives
+ * zeros.  FI_ERR_INVALID: null f, solution or heatmap, an unknown loc.  FI_ERR_RANGE: point or caller rows on a
+ * lattice of more than 2^31 - 1 nodes (their columns are int32, as in the triplet view). */
+FI_API int fi_field_error_map(fi_field* f, const float* solution /* N */, int32_t loc, float* heatmap /* N */,
+                              double* row_error_sums /* nullable, 3 */);
 
 /* ---- iso-surface helpers of the callers (SURVEY.md 8f rank 4): what the demo runs on every solved 2D field -------- */
 /* emilib::marching_squares (third_party/emilib/emilib/marching_squares.cpp:11-134) of `values - iso` — iso_surface,

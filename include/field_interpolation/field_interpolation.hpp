@@ -145,6 +145,19 @@ bool marching_cubes(const std::vector<int>& sizes, const float* values, float is
 bool sample_field(const std::vector<int>& sizes, const float* field, int64_t num_points, const float* positions, GradientKernel kernel,
                   bool want_gradients, std::vector<float>* values, std::vector<float>* gradients);
 
+/// Sum over rows of err^2 (err = rhs - row . solution in fp32, squared and summed in fp64), by kind of row: the
+/// least-squares objective the solve minimises, term by term.
+struct ErrorSums
+{
+	double model_rows = 0, point_rows = 0, caller_rows = 0;
+};
+
+/// generate_error_map of the field's own system, on the GPU and without its triplet list: bit-identical to
+/// generate_error_map(field->eq.triplets, solution, field->eq.rhs) of a materialised field, and also defined for
+/// deferred fields and systems beyond the int32 triplet view.  Rows appended to field->eq by hand are forwarded first,
+/// as the builders do.  fi_field_error_map (include/fi_b200.h) states the contract.  Returns {} on failure.
+std::vector<float> generate_error_map(LatticeField* field, const std::vector<float>& solution, ErrorSums* sums = nullptr);
+
 }  // namespace b200
 
 }  // namespace field_interpolation
