@@ -12,6 +12,7 @@ from .api import (FI_DEVICE, FI_F32, FI_F64, FI_HOST, FI_MIXED, FI_PRECOND_JACOB
                   kernel_launches, kernel_launches_reset, sdf_from_points, sdf_solve_cascade, solve_options,
                   solve_sparse_linear_exact, solve_sparse_linear_fast, solve_sparse_linear_with_guess,
                   solve_tiled_with_guess, upscale_field, bicubic_upsample, calc_area, iso_surface, marching_squares,
-                  marching_cubes, sample_field, generate_error_map)
+                  marching_cubes, sample_field, generate_error_map, nearest_point_distance,
+                  add_border_distance_constraints)
 
 __all__ = [n for n in dir() if not n.startswith("_")]

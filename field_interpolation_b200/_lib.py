@@ -81,6 +81,7 @@ SIGNATURES = {
     "fi_field_clone": (C.c_int, [_vp, _p(_vp)]),
     "fi_field_add_model": (C.c_int, [_vp, _p(fi_weights)]),
     "fi_field_add_points": (C.c_int, [_vp, _f, _i32, _f, _i32, _i64, _vp, _vp, _vp, _vp, _i32, _pi64]),
+    "fi_field_add_border_distance": (C.c_int, [_vp, _f, _i64, _vp, _i32, _pi64]),
     "fi_field_add_rows": (C.c_int, [_vp, _i64, _i64, _pi32, _pi32, _pf, _pf]),
     "fi_sdf_from_points": (C.c_int, [_i32, _pi32, _p(fi_weights), _i64, _vp, _vp, _vp, _i32, _p(_vp)]),
     "fi_field_counts": (C.c_int, [_vp, _pi64, _pi64]),
@@ -101,6 +102,7 @@ SIGNATURES = {
     "fi_bicubic_upsample": (C.c_int, [_i32, _i32, _vp, _i32, _vp, _i32]),
     "fi_marching_cubes": (C.c_int, [_pi32, _vp, _f, _i32, _vp, _vp, _i64, _vp, _i64, _pi64, _pi64]),
     "fi_sample_field": (C.c_int, [_i32, _pi32, _vp, _i64, _vp, _i32, _i32, _vp, _vp]),
+    "fi_nearest_point_distance": (C.c_int, [_i32, _i64, _vp, _i64, _vp, _i32, _vp, _vp]),
     "fi_sdf_solve_cascade": (C.c_int, [_i32, _pi32, _p(fi_weights), _i64, _vp, _vp, _vp, _p(fi_cascade_options), _vp, _i32,
                                        _p(fi_cascade_stats)]),
     "fi_comm_unique_id": (C.c_int, [_vp, _i64]),

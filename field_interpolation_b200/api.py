@@ -285,6 +285,25 @@ def add_rows(field: LatticeField, trip_row, trip_col, trip_val, rhs) -> None:
                                       v.ctypes.data_as(L._pf), b.ctypes.data_as(L._pf)))
 
 
+def add_border_distance_constraints(field: LatticeField, weight: float, positions) -> int:
+    """The border-distance rows of the reference's SDF caller (src/sdf_field.cpp:212-249; fi_field_add_border_distance,
+    include/fi_b200.h): for every border node, add_equation(weight, distance to the nearest position, node), in
+    ascending node order.  positions: (n, D) lattice coordinates, numpy array or CUDA tensor, n >= 1.  Returns the
+    number of rows appended (0 when weight == 0)."""
+    D = field.num_dim()
+    shape = tuple(positions.shape) if positions is not None else (0, D)
+    if len(shape) != 2 or shape[1] != D:
+        raise ValueError(f"positions must be (n, {D})")
+    if _is_device(positions):
+        positions = positions.contiguous()
+    n = int(shape[0])
+    p = _Buf(positions, n * D)
+    added = C.c_int64(0)
+    L.check(L.lib().fi_field_add_border_distance(field._h, float(weight), n, p.ptr, p.loc if p.loc is not None else FI_HOST,
+                                                 C.byref(added)))
+    return int(added.value)
+
+
 def sdf_from_points(sizes: Sequence[int], weights: Weights, positions, normals=None, point_weights=None) -> LatticeField:
     """field_interpolation.cpp:373-400."""
     D = len(sizes)
@@ -446,6 +465,35 @@ def sample_field(field, positions, gradient_kernel=None):
         L.check(L.lib().fi_sample_field(D, sizes, fb.ptr, N, pb.ptr, int(gradient_kernel) if want else 0, fb.loc, ptr(vals),
                                         ptr(grads) if want else None))
     return (vals, grads) if want else vals
+
+
+def nearest_point_distance(points, queries, want_index: bool = False):
+    """Distance from each query to the nearest of the points, and optionally that point's index
+    (fi_nearest_point_distance, include/fi_b200.h): bit-identical to the brute-force fp32 loop of the reference's SDF
+    caller.  points (n, D) and queries (m, D), D = 1..3, numpy arrays or CUDA tensors living in the same place.
+    Returns distances (m,) float32, or (distances, nearest (m,) int64) with want_index, living where the inputs live.
+    A query with no finite nearest distance reads +inf and index -1."""
+    pshape, qshape = tuple(points.shape), tuple(queries.shape)
+    if len(pshape) != 2 or len(qshape) != 2 or pshape[1] != qshape[1] or not 1 <= qshape[1] <= 3:
+        raise ValueError("points (n, D) and queries (m, D) with D = 1..3 are expected")
+    if _is_device(points) != _is_device(queries):
+        raise ValueError("points and queries must live in the same place (both host or both device)")
+    if _is_device(points):
+        points, queries = points.contiguous(), queries.contiguous()
+    D, n, m = int(qshape[1]), int(pshape[0]), int(qshape[0])
+    pb, qb = _Buf(points, n * D), _Buf(queries, m * D)
+    if pb.loc == FI_DEVICE:
+        import torch
+        dist = torch.empty(m, dtype=torch.float32, device=points.device)
+        idx = torch.empty(m, dtype=torch.int64, device=points.device) if want_index else None
+        ptr = lambda a: C.c_void_p(a.data_ptr())  # noqa: E731
+    else:
+        dist = np.empty(m, np.float32)
+        idx = np.empty(m, np.int64) if want_index else None
+        ptr = lambda a: C.c_void_p(a.ctypes.data)  # noqa: E731
+    if m:
+        L.check(L.lib().fi_nearest_point_distance(D, n, pb.ptr, m, qb.ptr, pb.loc, ptr(dist), ptr(idx) if want_index else None))
+    return (dist, idx) if want_index else dist
 
 
 def generate_error_map(field: LatticeField, solution, want_sums: bool = False):

@@ -721,6 +721,32 @@ int fi_field_add_rows(fi_field* f, int64_t num_rows, int64_t num_triplets, const
 	});
 }
 
+int fi_field_add_border_distance(fi_field* f, float weight, int64_t num_points, const float* positions, int32_t loc, int64_t* rows_added)
+{
+	return guarded([&] {
+		TraceScope trace("fi_field_add_border_distance");
+		if (rows_added) { *rows_added = 0; }
+		FI_REQUIRE(f != nullptr, FI_ERR_INVALID, "field is null");
+		FI_REQUIRE(loc == FI_HOST || loc == FI_DEVICE, FI_ERR_INVALID, "add_border_distance: unknown loc");
+		FI_REQUIRE(num_points >= 1, FI_ERR_INVALID, "add_border_distance: no points");
+		FI_REQUIRE(positions != nullptr, FI_ERR_INVALID, "positions is null");
+		FI_REQUIRE(num_points < (1ll << 32), FI_ERR_RANGE, "add_border_distance: 2^32 points or more");
+		FI_REQUIRE(f->g.N <= INT32_MAX, FI_ERR_RANGE, "add_border_distance: more than 2^31 - 1 nodes (columns are int32)");
+		if (weight == 0) { return; }  // add_equation drops the row
+		Staged<float> p(positions, static_cast<size_t>(num_points) * f->g.ndim, loc, f->stream);
+		HostRows&     R  = f->rows;
+		const int64_t r0 = R.rows();
+		append_border_rows(f->g, weight, num_points, p.ptr, R, f->stream);
+		Segment sg;
+		sg.kind = Segment::kRows;
+		sg.r0   = r0;
+		sg.r1   = R.rows();
+		f->segs.push_back(sg);
+		f->invalidate();
+		if (rows_added) { *rows_added = sg.r1 - sg.r0; }
+	});
+}
+
 int fi_sdf_from_points(int32_t ndim, const int32_t* sizes, const fi_weights* w, int64_t num_points, const float* positions,
                        const float* normals, const float* point_weights, int32_t loc, fi_field** out)
 {
@@ -1172,6 +1198,34 @@ int fi_sample_field(int32_t ndim, const int32_t* sizes, const float* field, int6
 		sample_field_device(g, num_points, p.ptr, x.ptr, gradient_kernel, values ? v.data() : nullptr, gradients ? gr.data() : nullptr, s);
 		if (values) { FI_CUDA(cudaMemcpy(values, v.data(), np * sizeof(float), cudaMemcpyDeviceToHost)); }
 		if (gradients) { FI_CUDA(cudaMemcpy(gradients, gr.data(), nd * sizeof(float), cudaMemcpyDeviceToHost)); }
+	});
+}
+
+int fi_nearest_point_distance(int32_t ndim, int64_t num_points, const float* points, int64_t num_queries, const float* queries, int32_t loc,
+                              float* distances, int64_t* nearest)
+{
+	return guarded([&] {
+		TraceScope trace("fi_nearest_point_distance");
+		FI_REQUIRE(1 <= ndim && ndim <= kMaxDim, FI_ERR_INVALID, "nearest_point_distance: ndim must be 1..3");
+		FI_REQUIRE(loc == FI_HOST || loc == FI_DEVICE, FI_ERR_INVALID, "nearest_point_distance: unknown loc");
+		FI_REQUIRE(num_points >= 0 && num_queries >= 0, FI_ERR_INVALID, "nearest_point_distance: negative count");
+		FI_REQUIRE(num_points == 0 || points, FI_ERR_INVALID, "nearest_point_distance: points is null");
+		FI_REQUIRE(num_queries == 0 || queries, FI_ERR_INVALID, "nearest_point_distance: queries is null");
+		FI_REQUIRE(num_points < (1ll << 32), FI_ERR_RANGE, "nearest_point_distance: 2^32 points or more");
+		if (num_queries == 0 || (!distances && !nearest)) { return; }
+		const size_t  nq = static_cast<size_t>(num_queries);
+		cudaStream_t  s  = nullptr;
+		Staged<float> p(points, static_cast<size_t>(num_points) * ndim, loc, s), q(queries, nq * ndim, loc, s);
+		if (loc == FI_DEVICE) {
+			nearest_points_device(ndim, num_points, p.ptr, num_queries, q.ptr, distances, nearest, s);
+			return;
+		}
+		DevBuf<float>   d(distances ? nq : 0);
+		DevBuf<int64_t> k(nearest ? nq : 0);
+		nearest_points_device(ndim, num_points, p.ptr, num_queries, q.ptr, distances ? d.data() : nullptr, nearest ? k.data() : nullptr, s);
+		if (distances) { FI_CUDA(cudaMemcpyAsync(distances, d.data(), nq * sizeof(float), cudaMemcpyDeviceToHost, s)); }
+		if (nearest) { FI_CUDA(cudaMemcpyAsync(nearest, k.data(), nq * sizeof(int64_t), cudaMemcpyDeviceToHost, s)); }
+		FI_CUDA(cudaStreamSynchronize(s));
 	});
 }
 

@@ -1373,3 +1373,5 @@ template bool apply_data_term<double>(const Geom&, const DataTerm<double>&, cons
 #include "sample_field.cuh"
 // So does the error map of a field's own system (bit-identical to generate_error_map on its exported triplets).
 #include "field_error_map.cuh"
+// So does the exact nearest-point search (bit-identical to the brute-force loop of the reference's SDF caller).
+#include "nearest_points.cuh"

@@ -198,6 +198,16 @@ void    point_error_map(const Geom& g, PointView pv, int64_t p0, int64_t p1, con
 void    caller_rows_error_map(const Geom& g, const HostRows& rows, int64_t r0, int64_t r1, const float* d_x, float* d_heat, double* d_sum,
                               ErrorMapScratch& sc, cudaStream_t s);
 
+// ---- nearest_points.cuh (included by assembly.cu, compiled with -fmad=false) ----------------------------------
+// Exact nearest-point search; fi_nearest_point_distance states the contract.  Each call builds its search structure
+// from the cloud (n_points interleaved points of ndim floats, device) and frees it.
+// d_dist (nullable) and d_nearest (nullable; -1 where the distance is +inf) hold one entry per query.
+void nearest_points_device(int ndim, int64_t n_points, const float* d_points, int64_t n_queries, const float* d_queries, float* d_dist,
+                           int64_t* d_nearest, cudaStream_t s);
+// Appends to `rows` the border-distance rows of the reference's SDF caller: one row (node, 1.0f * weight), rhs
+// distance * weight, per border node of g in ascending linear index (fi_field_add_border_distance).
+void append_border_rows(const Geom& g, float weight, int64_t n_points, const float* d_points, HostRows& rows, cudaStream_t s);
+
 // ---- errormap.cu ------------------------------------------------------------------------------------------
 void error_map(int64_t nt, const fi_triplet* h_trips, int64_t n, const float* h_x, int64_t nrows, const float* h_rhs, float* h_out);
 

@@ -279,6 +279,28 @@ std::vector<float> generate_error_map(LatticeField* field, const std::vector<flo
 	return heat;
 }
 
+long long add_border_distance_constraints(LatticeField* field, float weight, int num_points, const float positions[])
+{
+	if (field == nullptr) { return -1; }
+	return build(field, [&](fi_field* h) { return fi_field_add_border_distance(h, weight, num_points, positions, FI_HOST, nullptr); });
+}
+
+bool nearest_point_distance(int ndim, int64_t num_points, const float* points, int64_t num_queries, const float* queries,
+                            std::vector<float>* distances, std::vector<int64_t>* nearest)
+{
+	if (distances == nullptr || num_queries < 0) { return false; }
+	distances->clear();
+	if (nearest) { nearest->clear(); }
+	std::vector<float>   d(static_cast<size_t>(num_queries));
+	std::vector<int64_t> k(nearest ? static_cast<size_t>(num_queries) : 0);
+	if (fi_nearest_point_distance(ndim, num_points, points, num_queries, queries, FI_HOST, d.data(), nearest ? k.data() : nullptr) != FI_OK) {
+		return false;
+	}
+	*distances = std::move(d);
+	if (nearest) { *nearest = std::move(k); }
+	return true;
+}
+
 }  // namespace b200
 
 using b200::build;

@@ -29,7 +29,8 @@ extern "C" {
 /* 4: + fi_marching_cubes (additions only) */
 /* 5: + fi_sample_field (additions only) */
 /* 6: + fi_field_error_map (additions only) */
-#define FI_B200_ABI_VERSION 6
+/* 7: + fi_nearest_point_distance, fi_field_add_border_distance (additions only) */
+#define FI_B200_ABI_VERSION 7
 
 #if defined(__GNUC__)
 #define FI_API __attribute__((visibility("default")))
@@ -151,6 +152,23 @@ FI_API int fi_field_add_points(fi_field* f, float value_weight, int32_t value_ke
  * trip_row in [0,num_rows) non-decreasing, trip_col in [0,N).  Host buffers. */
 FI_API int fi_field_add_rows(fi_field* f, int64_t num_rows, int64_t num_triplets, const int32_t* trip_row,
                       const int32_t* trip_col, const float* trip_val, const float* rhs);
+
+/* The border-distance rows of the reference's SDF caller, generate_sdf_field (src/sdf_field.cpp:212-249), generalised to
+ * D dimensions: for every lattice node on the border (some coordinate c_d is 0 or n_d - 1; axes of 1 or 2 nodes make
+ * every node a border node), in ascending linear index (x fastest), the row of
+ *   add_equation(weight, {sqrt(min_i |p_i - q|^2)}, {{node, 1.0f}})
+ * with q the node's integer coordinates as floats and the distance exactly as fi_nearest_point_distance computes it:
+ * one triplet (row, node, 1.0f * weight) and rhs distance * weight (reference sparse_linear.cpp:34-50, restated in
+ * host/sparse_linear.cpp:40-51).  positions: num_points x D floats in lattice coordinates, as fi_field_add_points takes them, living where `loc` says (device buffers need
+ * 4-byte alignment only).  The rows are stored as caller rows, so fi_field_export of the field is bit-identical to
+ * the same builder calls with the caller's brute-force loop and add_equation, in every order of calls.  weight == 0
+ * appends nothing (as add_equation); negative and NaN weights append.  A cloud whose points all have a non-finite
+ * coordinate appends rows with rhs +inf * weight, as the loop does.  rows_added (nullable) receives the number of
+ * rows appended.  FI_ERR_INVALID: null f or positions, num_points < 1 (the loop would give every row an infinite
+ * rhs), an unknown loc.  FI_ERR_RANGE: a lattice of more than 2^31 - 1 nodes (columns are int32), 2^32 points or
+ * more.  The lattice's border distances are the only data that cross to the host (4 B per border node). */
+FI_API int fi_field_add_border_distance(fi_field* f, float weight, int64_t num_points, const float* positions, int32_t loc,
+                                        int64_t* rows_added);
 
 /* sdf_from_points, field_interpolation.cpp:373-400 = create + add_model + add_points. */
 FI_API int fi_sdf_from_points(int32_t ndim, const int32_t* sizes, const fi_weights* w, int64_t num_points,
@@ -288,6 +306,27 @@ FI_API int fi_marching_cubes(const int32_t* sizes /* 3 */, const float* values, 
 FI_API int fi_sample_field(int32_t ndim, const int32_t* sizes, const float* field, int64_t num_points,
                            const float* positions /* D per point, lattice coordinates */, int32_t gradient_kernel,
                            int32_t loc, float* values /* nullable */, float* gradients /* D per point, nullable */);
+
+/* Exact nearest-point search on the device: for each query q (D = ndim floats), the distance to the nearest of the
+ * points and that point's index, bit-identical to the brute-force loop of the reference's SDF caller
+ * (src/sdf_field.cpp:212-249), in fp32 without FMA contraction:
+ *   dx_d = p_i[d] - q[d];  d2_i = dx_0 * dx_0 + dx_1 * dx_1 (+ dx_2 * dx_2), summed left to right
+ *   closest = +inf;  for i in order: closest = d2_i < closest ? d2_i : closest      (std::min(closest, d2_i))
+ *   distances[j] = sqrt(closest), correctly rounded
+ *   nearest[j]   = the smallest i with d2_i == closest, or -1 when closest is +inf
+ * A NaN d2 never wins, so points with a non-finite coordinate never win; a non-finite query, or a cloud without a
+ * finite point, gives +inf and -1.  Ties, duplicate points, points anywhere (inside or outside any lattice) and
+ * subnormal differences all follow the loop.  Each call builds its search structure from the points (an implicit
+ * box tree over their Morton order) and frees it.  Use it to measure how far mesh vertices or samples lie from the
+ * input cloud (the one-sided Hausdorff distance of a reconstruction) and to find each one's corresponding point.
+ * points (num_points x D), queries (num_queries x D), distances (nullable, num_queries floats) and nearest (nullable,
+ * num_queries int64) live where `loc` says; device buffers need 4-byte alignment only (8 for nearest).  Both outputs
+ * null, or num_queries == 0, is a no-op; num_points == 0 gives +inf and -1 everywhere.  FI_ERR_INVALID: ndim
+ * outside 1..3, an unknown loc, a negative count, null points or queries with a positive count.  FI_ERR_RANGE: 2^32
+ * points or more. */
+FI_API int fi_nearest_point_distance(int32_t ndim, int64_t num_points, const float* points, int64_t num_queries,
+                                     const float* queries, int32_t loc, float* distances /* nullable */,
+                                     int64_t* nearest /* nullable */);
 
 /* Coarse-to-fine solve mirroring the demo's recipe (src/sdf_field.cpp:251-304) applied recursively:
  * positions are in UNIT coordinates and are scaled per level by (size-1) as on_lattice does (:198-210);

@@ -158,6 +158,21 @@ struct ErrorSums
 /// as the builders do.  fi_field_error_map (include/fi_b200.h) states the contract.  Returns {} on failure.
 std::vector<float> generate_error_map(LatticeField* field, const std::vector<float>& solution, ErrorSums* sums = nullptr);
 
+/// The border-distance rows of the reference's SDF caller (src/sdf_field.cpp:212-249): for every lattice node on the
+/// border, in ascending index, add_equation(&field->eq, Weight{weight}, {sqrt(closest)}, {{node, 1.0f}}) with closest
+/// the smallest fp32 squared distance from the node to the positions (lattice coordinates, D interleaved floats each).
+/// The search runs on the GPU; the rows are bit-identical to that loop's.  Rows appended to field->eq by hand are
+/// forwarded first, and the new rows are mirrored into field->eq unless triplets are deferred, as the builders do.
+/// fi_field_add_border_distance (include/fi_b200.h) states the contract.  Returns the number of rows appended, or -1
+/// on failure (num_points < 1 included).
+long long add_border_distance_constraints(LatticeField* field, float weight, int num_points, const float positions[]);
+
+/// Distance from each query to the nearest point, and (nearest != nullptr) that point's index, on the GPU:
+/// bit-identical to the brute-force fp32 loop of the reference's SDF caller.  points and queries hold ndim interleaved
+/// floats each.  fi_nearest_point_distance (include/fi_b200.h) states the contract.  Returns false on failure.
+bool nearest_point_distance(int ndim, int64_t num_points, const float* points, int64_t num_queries, const float* queries,
+                            std::vector<float>* distances, std::vector<int64_t>* nearest = nullptr);
+
 }  // namespace b200
 
 }  // namespace field_interpolation
