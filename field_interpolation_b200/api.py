@@ -202,12 +202,13 @@ class LatticeField:
         return (out if _is_device(out) else o.keep), st.as_dict()
 
     def time_iterations(self, iterations: int, options: Optional[L.fi_solve_options] = None):
-        """Device ms (totals over `iterations` launches): whole iterations, apply kernels, update, direction; fused?"""
+        """Device ms (totals over `iterations` launches): whole iterations, apply kernels, update, direction; fused?;
+        x_ring: iterations per x update of the solve (the ring of directions it kept; 1 for the unfused iteration)"""
         opt = options if options is not None else solve_options()
         ms = (C.c_double * 8)()
         L.check(L.lib().fi_field_time_iterations(self._h, C.byref(opt), int(iterations), ms))
         return {"iteration_ms": ms[0], "apply_ms": ms[1], "update_ms": ms[2], "direction_ms": ms[3], "fused": bool(ms[4]),
-                "stencil_ms": ms[5], "data_term_ms": ms[6]}
+                "stencil_ms": ms[5], "data_term_ms": ms[6], "x_ring": int(ms[7])}
 
 
 # ---- builders (field_interpolation.hpp:116-173) ------------------------------------------------------

@@ -6,10 +6,15 @@
 // converge (the last iterate is returned).  A^T A is symmetric positive (semi-)definite, so CG replaces
 // Eigen's BiCGSTAB at half the operator applications per iteration.
 //
-// x is not needed by the iteration itself, and the fused path keeps the last two directions (p ping-pongs between two
-// buffers), so x is updated every SECOND iteration with both terms, x += a_k p_k + a_{k+1} p_{k+1}: the even iteration moves
-// 16 B/cell (q, r, M read, r written), the odd one 32 B/cell — 24 on average instead of 28; an odd iteration count is
-// completed by one flush after the loop.  (kXClassic / kXSkip / kXBoth below.)
+// x is not needed by the iteration itself, so the fused path keeps a ring of the last m directions (iteration k reads p_k-1
+// from PcgWork::dir[k mod m] and writes p_k to dir[(k+1) mod m]) and updates x once per m iterations with all m terms.
+// Iterations k mod m < m-1 are the *skip* form: they park a_k in PcgWork::alpha and move 16 B/cell (q, r, M read, r
+// written).  Iteration k mod m = m-1 is the *flush* form: x += s with s = a_k-m+1 p_k-m+1, then s += a_j p_j for j up to k in
+// increasing order, which moves (m+6) words per cell.  Averaged over m iterations that is 4 (5 + 2/m) bytes per fp32 cell:
+// 24 at m = 2, 21 at m = 8, against 28 for x += a p every iteration.  The directions still pending when the loop stops are
+// flushed by one launch after it.  m is chosen per solve by choose_x_ring.  Slab-sharded solves keep the two-direction
+// scheme of the peer and NCCL update kernels (kXSkip / kXBoth below: a_k parked in PcgState::alpha_prev, both terms applied
+// by the odd iteration).
 // Per iteration three kernels touch the lattice vectors:
 //   apply      q = (S+P) p, p.q                      read p, write q              8 B/cell (fp32)
 //   update     x += a p, r -= a q, r.Mr, r.r         read x,p,q,r,M, write x,r   28 B/cell
@@ -278,6 +283,106 @@ __global__ void __launch_bounds__(kThreads) pcg_update_kernel(int64_t n, T* __re
 	});
 }
 
+// Directions of a flush, oldest first (by value: a kernel argument).
+template <typename T>
+struct DirRing
+{
+	const T* p[kMaxXRing];
+};
+
+// r -= a q with the two dot products, and for M > 0 (flush form) also x += a[0] d_0 + ... + a[M-1] d_M-1, summed in that order
+// into a temporary that is added to x last.
+template <typename T, int M, bool PACKED>
+__device__ __forceinline__ void ring_update_elements(int64_t k, T* __restrict__ x, T* __restrict__ r, const DirRing<T>& d, const T* __restrict__ q,
+                                                     const T* __restrict__ minv, T alpha, const T (&a)[kMaxXRing], double (&acc)[2])
+{
+	using P         = typename Pack<T>::type;
+	constexpr int V = PACKED ? Pack<T>::V : 1;
+	constexpr int MD = M > 0 ? M : 1;
+	T ra[V], qa[V], ma[V], xa[V], da[MD][V];
+	if (PACKED) {
+		*reinterpret_cast<P*>(ra) = reinterpret_cast<const P*>(r)[k];
+		*reinterpret_cast<P*>(qa) = reinterpret_cast<const P*>(q)[k];
+		*reinterpret_cast<P*>(ma) = reinterpret_cast<const P*>(minv)[k];
+		if (M > 0) {
+			*reinterpret_cast<P*>(xa) = reinterpret_cast<const P*>(x)[k];
+#pragma unroll
+			for (int j = 0; j < M; ++j) { *reinterpret_cast<P*>(da[j]) = reinterpret_cast<const P*>(d.p[j])[k]; }
+		}
+	} else {
+		ra[0] = r[k];
+		qa[0] = q[k];
+		ma[0] = minv[k];
+		if (M > 0) {
+			xa[0] = x[k];
+#pragma unroll
+			for (int j = 0; j < M; ++j) { da[j][0] = d.p[j][k]; }
+		}
+	}
+#pragma unroll
+	for (int e = 0; e < V; ++e) {
+		if (M > 0) {
+			T s = a[0] * da[0][e];
+#pragma unroll
+			for (int j = 1; j < M; ++j) { s += a[j] * da[j][e]; }
+			xa[e] += s;
+		}
+		ra[e] -= alpha * qa[e];
+		const double rd = static_cast<double>(ra[e]);
+		acc[0] += rd * static_cast<double>(ma[e] * ra[e]);
+		acc[1] += rd * rd;
+	}
+	if (PACKED) {
+		if (M > 0) { reinterpret_cast<P*>(x)[k] = *reinterpret_cast<const P*>(xa); }
+		reinterpret_cast<P*>(r)[k] = *reinterpret_cast<const P*>(ra);
+	} else {
+		if (M > 0) { x[k] = xa[0]; }
+		r[k] = ra[0];
+	}
+}
+
+// The update kernel of the unsharded fused iteration with a ring of m directions (header comment).  M = 0: skip form, x is
+// left alone and a_k is parked in alpha[pos] (pos = k mod m).  M = m: flush form, d holds p_k-m+1 .. p_k and alpha[0 .. m-2]
+// the parked step lengths of the first m-1 of them.
+template <typename T, int M>
+__global__ void __launch_bounds__(kThreads) pcg_update_ring_kernel(int64_t n, T* __restrict__ x, T* __restrict__ r, DirRing<T> d,
+                                                                   const T* __restrict__ q, const T* __restrict__ minv, PcgState* st, int par,
+                                                                   double* __restrict__ alpha, int pos, double* partial, unsigned* ticket)
+{
+	__shared__ double red[32];
+	if (st->done) { return; }
+	const double pq = st->pq;
+	if (!(pq > 0.0)) {  // breakdown (singular direction or NaN): keep the last iterate
+		if (blockIdx.x == 0 && threadIdx.x == 0) {
+			st->breakdown = 1;
+			st->done      = 1;
+		}
+		return;
+	}
+	const double alpha_d = st->rho[par] / pq;
+	T            a[kMaxXRing];
+#pragma unroll
+	for (int j = 0; j < kMaxXRing; ++j) { a[j] = j < M - 1 ? static_cast<T>(alpha[j]) : T(0); }
+	if (M > 0) { a[M > 0 ? M - 1 : 0] = static_cast<T>(alpha_d); }
+	double acc[2] = {0, 0};
+	for_each_pack<T>(n, [&](int64_t k, bool packed) {
+		if (packed) {
+			ring_update_elements<T, M, true>(k, x, r, d, q, minv, static_cast<T>(alpha_d), a, acc);
+		} else {
+			ring_update_elements<T, M, false>(k, x, r, d, q, minv, static_cast<T>(alpha_d), a, acc);
+		}
+	});
+	acc[0] = block_sum(acc[0], red);
+	acc[1] = block_sum(acc[1], red);
+	grid_sum<2>(acc, partial, ticket, red, [&](const double(&tot)[2]) {
+		if (M == 0) { alpha[pos] = alpha_d; }
+		st->rho[par ^ 1] = tot[0];
+		st->rr           = tot[1];
+		st->iters += 1;
+		if (tot[1] <= st->tol2bb || st->iters >= st->max_iters || !(tot[0] > 0.0)) { st->done = 1; }
+	});
+}
+
 // The update kernel of a slab on the peer-memory path: waits for the all-reduced p.Ap in its mailbox, updates x
 // and r, stores the boundary planes of the new r straight into the neighbours' halo planes (NVLink peer stores),
 // and the last block publishes this slab's (r.Mr, r.r) to every rank.
@@ -457,13 +562,82 @@ __global__ void add_f32_f64_kernel(int64_t n, const float* __restrict__ e, doubl
 	for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += stride) { x[i] += static_cast<double>(e[i]); }
 }
 
-// x += alpha_prev * p: completes an odd number of iterations of the deferred x update
+// x += alpha[0] d_0 + ... + alpha[count-1] d_count-1 (1 <= count < kMaxXRing), summed in the order of the flush form: the x
+// update of the iterations still pending when the loop stopped
 template <typename T>
-__global__ void __launch_bounds__(kThreads) pcg_flush_x_kernel(int64_t n, T* __restrict__ x, const T* __restrict__ p, const PcgState* st)
+__global__ void __launch_bounds__(kThreads) pcg_flush_x_kernel(int64_t n, T* __restrict__ x, DirRing<T> d, const double* alpha, int count)
 {
-	const T       a      = static_cast<T>(st->alpha_prev);
+	T a[kMaxXRing];
+#pragma unroll
+	for (int j = 0; j < kMaxXRing; ++j) { a[j] = j < count ? static_cast<T>(alpha[j]) : T(0); }
 	const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
-	for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += stride) { x[i] += a * p[i]; }
+	for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += stride) {
+		T s = a[0] * d.p[0][i];
+#pragma unroll
+		for (int j = 1; j < kMaxXRing; ++j) {
+			if (j < count) { s += a[j] * d.p[j][i]; }
+		}
+		x[i] += s;
+	}
+}
+
+// How many directions the fused iteration keeps before it updates x (header comment): FI_B200_X_RING=2|4|8 when set, else
+// kDefaultXRing; 2 where the two-direction working set (x, r, q, M^-1 and two directions) fits the L2 cache — extra buffers
+// there would push the vectors out of it for a few bytes per cell — or where no fused kernel runs; halved while the buffers
+// not yet allocated would take more than half of the free device memory.  8 measured best on a B200 at 512^3 and 1024^3:
+// 512^3 fp32 iteration 0.998 / 0.948 / 0.937 ms at m = 2 / 4 / 8 (DESIGN.md §3, profiles/x_ring_b200.jsonl).
+constexpr int kDefaultXRing = 8;
+
+template <typename T>
+int choose_x_ring(const Operator<T>& op)
+{
+	const bool fusable = op.g.ndim >= 2 && !op.g.tile && op.use_fast != kStencilGeneric && op.dist == nullptr && !op.g.sharded();
+	if (!fusable) { return 2; }
+	const char* env = std::getenv("FI_B200_X_RING");
+	int         m   = kDefaultXRing;
+	const size_t vec = static_cast<size_t>(op.g.N) * sizeof(T);
+	if (env && *env) {
+		m = std::atoi(env);
+		FI_REQUIRE(m == 2 || m == 4 || m == 8, FI_ERR_INVALID, "FI_B200_X_RING must be 2, 4 or 8");
+	} else {
+		int dev = 0, l2 = 0;
+		FI_CUDA(cudaGetDevice(&dev));
+		FI_CUDA(cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, dev));
+		const size_t l2_bytes = l2 > 0 ? static_cast<size_t>(l2) : static_cast<size_t>(126) << 20;  // unreported: the B200's
+		if (6 * vec <= l2_bytes) { return 2; }
+	}
+	size_t free_b = 0, total_b = 0;
+	FI_CUDA(cudaMemGetInfo(&free_b, &total_b));
+	while (m > 2 && static_cast<size_t>(std::max(0, m - op.work.dirs)) * vec > free_b / 2) { m /= 2; }
+	return m;
+}
+
+// dir[0 .. m) allocated; the new ones zeroed (a flush timed on its own reads every slot)
+template <typename T>
+void ensure_ring(PcgWork<T>& w, size_t n, int m, cudaStream_t s)
+{
+	for (; w.dirs < m; ++w.dirs) {
+		w.dir[w.dirs].resize(n);
+		w.dir[w.dirs].zero(s);
+	}
+}
+
+// Launches the update of ring position pos (= k mod m) of the unsharded fused iteration: the skip form, or at pos = m-1 the
+// flush form over p_k-m+1 .. p_k, which sit in dir[1], ..., dir[m-1], dir[0].
+template <typename T>
+void launch_ring_update(PcgWork<T>& w, int m, int pos, int grid, int64_t n, T* x, const T* minv, int par, cudaStream_t s)
+{
+	DirRing<T> d = {};
+	if (pos < m - 1) {
+		auto ku = pcg_update_ring_kernel<T, 0>;
+		FI_LAUNCH(ku, grid, kThreads, 0, s, n, x, w.r.data(), d, w.q.data(), minv, w.state.data(), par, w.alpha.data(), pos, w.partial.data(),
+		          w.ticket.data());
+		return;
+	}
+	for (int j = 0; j < m; ++j) { d.p[j] = w.dir[(j + 1) % m].data(); }
+	auto ku = m == 8 ? pcg_update_ring_kernel<T, 8> : m == 4 ? pcg_update_ring_kernel<T, 4> : pcg_update_ring_kernel<T, 2>;
+	FI_LAUNCH(ku, grid, kThreads, 0, s, n, x, w.r.data(), d, w.q.data(), minv, w.state.data(), par, w.alpha.data(), pos, w.partial.data(),
+	          w.ticket.data());
 }
 
 template <typename T>
@@ -473,15 +647,15 @@ void ensure_work(Operator<T>& op, cudaStream_t s)
 	const size_t n = static_cast<size_t>(op.g.N);
 	if (w.r.size() != n) {
 		w.r.resize(n);
-		w.p.resize(n);
 		w.q.resize(n);
-		w.p2.resize(n);
 		// the fused stencil kernel reads p_old before the first direction exists (times beta = 0): it must be finite.  On a slab
 		// the halo planes and the planes beyond the lattice of r and q are read too; elsewhere every element of r and q is
 		// written before it is read.  (On the solver's own stream: it is non-blocking, so work on the null stream is not
-		// ordered with it.)
-		w.p.zero(s);
-		w.p2.zero(s);
+		// ordered with it.)  Directions beyond the first two are allocated by the solve that needs them (ensure_ring).
+		for (int j = 2; j < kMaxXRing; ++j) { w.dir[j].release(); }
+		w.dirs = 0;
+		ensure_ring(w, n, 2, s);
+		w.alpha.resize(kMaxXRing - 1);
 		if (op.g.sharded()) {
 			w.r.zero(s);
 			w.q.zero(s);
@@ -577,8 +751,12 @@ PcgResult pcg_solve(Operator<T>& op, const T* b, T* x, double tol, long long max
 		max_iter = 2 * static_cast<long long>(op.g.size[0]) * op.g.size[1] * op.g.size[2];
 	}
 	if (!(tol > 0)) { tol = std::is_same<T, float>::value ? 1.1920929e-07 : 2.220446049250313e-16; }
-	check_every = std::max(2, check_every <= 0 ? 32 : check_every);
-	check_every += check_every & 1;  // whole parity pairs per graph
+	// directions kept per x update of the fused iteration (2 on a slab: the peer and NCCL update kernels ping-pong)
+	const int ring = choose_x_ring(op);
+	ensure_ring(w, static_cast<size_t>(op.g.N), ring, s);
+	// whole rings per graph: graph slot i is then always ring position i mod m (and parity i & 1)
+	check_every = std::max(ring, check_every <= 0 ? 32 : check_every);
+	check_every = (check_every + ring - 1) / ring * ring;
 
 	cudaEvent_t e0, e1;
 	FI_CUDA(cudaEventCreate(&e0));
@@ -606,8 +784,9 @@ PcgResult pcg_solve(Operator<T>& op, const T* b, T* x, double tol, long long max
 		op.apply(x, w.q.data(), nullptr, nullptr, s);
 	}
 	{
+		// p goes to dir[0]: the p_old of iteration 0 (read times beta = 0)
 		auto kern = pcg_init_kernel<T>;
-		FI_LAUNCH(kern, grid, kThreads, 0, s, n, rhs + off, zero_guess ? static_cast<const T*>(nullptr) : w.q.data() + off, op.minv.data() + off, r_vec + off, w.p.data() + off,
+		FI_LAUNCH(kern, grid, kThreads, 0, s, n, rhs + off, zero_guess ? static_cast<const T*>(nullptr) : w.q.data() + off, op.minv.data() + off, r_vec + off, w.dir[0].data() + off,
 		          w.state.data(), tol, max_iter, w.partial.data(), w.ticket.data(), dist ? 1 : 0);
 		if (dist) {
 			dist->allreduce(w.state.data()->part, 3, s);
@@ -628,7 +807,6 @@ PcgResult pcg_solve(Operator<T>& op, const T* b, T* x, double tol, long long max
 		const int* d_done = &w.state.data()->done;
 		double*    d_pq   = &w.state.data()->pq;
 		// check_every iterations per convergence poll
-		T*   pp[2] = {w.p.data(), w.p2.data()};
 		// every solve gets its own block of mailbox sequence numbers (all ranks count solves alike)
 		const unsigned long long seq_base = link ? (dist->next_seq() << 40) : 0ull;
 		// Who publishes p.Ap and who ends the iteration on the peer-memory path (FI_B200_PEER_FOLD, the same on every rank):
@@ -647,12 +825,14 @@ PcgResult pcg_solve(Operator<T>& op, const T* b, T* x, double tol, long long max
 		// with the grid-stride walk, 1.398 ms blocked (r2k / r2m).  FI_B200_PEER_UPDATE=blocked|stride overrides.
 		const char* walk_env = std::getenv("FI_B200_PEER_UPDATE");
 		const bool  peer_update_blocked = walk_env ? walk_env[0] == 'b' : n < (48ll << 20);
-		bool deferred_x = false;  // the fused path updates x every second iteration (kXSkip / kXBoth)
+		bool deferred_x = false;  // the fused path updates x once per ring of directions
 		auto enqueue_round = [&] {
 			for (int it = 0; it < check_every; ++it) {
-				const int par = it & 1;
-				// fused form: direction update folded into the stencil's load stage (p ping-pongs between two buffers)
-				const bool fused = stencil_fused_step<T>(op.use_fast, op.g, op.tabs, r_vec, op.minv.data(), pp[par], pp[par ^ 1], w.q.data(),
+				const int par = it & 1, pos = it % ring;
+				// fused form: direction update folded into the stencil's load stage (p_old = dir[pos], p_new = dir[pos + 1 mod m])
+				T* const   p_old = w.dir[pos].data();
+				T* const   p_new = w.dir[(pos + 1) % ring].data();
+				const bool fused = stencil_fused_step<T>(op.use_fast, op.g, op.tabs, r_vec, op.minv.data(), p_old, p_new, w.q.data(),
 				                                         w.state.data(), par, d_pq, op.partial.data(), op.ticket.data(), d_done, s);
 				deferred_x = deferred_x || fused;
 				if (fused && link) {
@@ -663,19 +843,22 @@ PcgResult pcg_solve(Operator<T>& op, const T* b, T* x, double tol, long long max
 					pub.par   = par;
 					pub.base  = seq_base;
 					pub.st    = w.state.data();
-					const bool published = apply_data_term<T>(op.g, op.data, pp[par ^ 1], w.q.data(), d_pq, d_done, s, data_publishes ? &pub : nullptr);
+					const bool published = apply_data_term<T>(op.g, op.data, p_new, w.q.data(), d_pq, d_done, s, data_publishes ? &pub : nullptr);
 					const bool in_update = fold_mode == 1;
 					if (!published && !in_update) { FI_LAUNCH(peer_publish_kernel, 1, 32, 0, s, *link, 0, par, seq_base, w.state.data(), d_pq, 1, d_done); }
 					auto ku = par == 0 ? pcg_update_peer_kernel<T, kXSkip> : pcg_update_peer_kernel<T, kXBoth>;
-					FI_LAUNCH(ku, grid, kThreads, 0, s, n, x + off, r_vec + off, pp[par ^ 1] + off, pp[par] + off, w.q.data() + off, op.minv.data() + off,
+					FI_LAUNCH(ku, grid, kThreads, 0, s, n, x + off, r_vec + off, p_new + off, p_old + off, w.q.data() + off, op.minv.data() + off,
 					          w.state.data(), par, w.partial.data(), w.ticket.data(), *link, push, seq_base, (in_update ? 1 : 0) | (update_finishes ? 2 : 0),
 					          peer_update_blocked ? 1 : 0);
 					if (!update_finishes) { FI_LAUNCH(pcg_update_finish_peer_kernel, 1, 32, 0, s, w.state.data(), par, *link, seq_base); }
+				} else if (fused && !dist) {
+					apply_data_term<T>(op.g, op.data, p_new, w.q.data(), d_pq, d_done, s);
+					launch_ring_update<T>(w, ring, pos, grid, n, x, op.minv.data(), par, s);
 				} else if (fused) {
-					apply_data_term<T>(op.g, op.data, pp[par ^ 1], w.q.data(), d_pq, d_done, s);
+					apply_data_term<T>(op.g, op.data, p_new, w.q.data(), d_pq, d_done, s);
 					if (dist) { dist->allreduce(d_pq, 1, s); }
 					auto ku = par == 0 ? pcg_update_kernel<T, kXSkip> : pcg_update_kernel<T, kXBoth>;
-					FI_LAUNCH(ku, grid, kThreads, 0, s, n, x + off, r_vec + off, pp[par ^ 1] + off, pp[par] + off, w.q.data() + off, op.minv.data() + off,
+					FI_LAUNCH(ku, grid, kThreads, 0, s, n, x + off, r_vec + off, p_new + off, p_old + off, w.q.data() + off, op.minv.data() + off,
 					          w.state.data(), par, w.partial.data(), w.ticket.data(), dist ? 1 : 0);
 					if (dist) {
 						dist->allreduce(w.state.data()->part, 2, s);
@@ -684,12 +867,13 @@ PcgResult pcg_solve(Operator<T>& op, const T* b, T* x, double tol, long long max
 					}
 				} else {
 					FI_REQUIRE(dist == nullptr, FI_ERR_UNSUPPORTED, "a slab-sharded solve needs the fused 3D stencil kernel");
-					op.apply(w.p.data(), w.q.data(), d_pq, d_done, s);
+					T* const p = w.dir[0].data();
+					op.apply(p, w.q.data(), d_pq, d_done, s);
 					auto ku = pcg_update_kernel<T, kXClassic>;
-					FI_LAUNCH(ku, grid, kThreads, 0, s, n, x, w.r.data(), w.p.data(), static_cast<const T*>(nullptr), w.q.data(), op.minv.data(), w.state.data(), par,
+					FI_LAUNCH(ku, grid, kThreads, 0, s, n, x, w.r.data(), p, static_cast<const T*>(nullptr), w.q.data(), op.minv.data(), w.state.data(), par,
 					          w.partial.data(), w.ticket.data(), 0);
 					auto kd = pcg_direction_kernel<T>;
-					FI_LAUNCH(kd, grid, kThreads, 0, s, n, w.r.data(), op.minv.data(), w.p.data(), w.state.data(), par);
+					FI_LAUNCH(kd, grid, kThreads, 0, s, n, w.r.data(), op.minv.data(), p, w.state.data(), par);
 				}
 			}
 		};
@@ -739,11 +923,18 @@ PcgResult pcg_solve(Operator<T>& op, const T* b, T* x, double tol, long long max
 			cudaGraphExecDestroy(exec);
 			cudaGraphDestroy(graph);
 		}
-		if (deferred_x && (h.iters & 1)) {
-			// an odd number of iterations ran: the last one (even-numbered) parked its x update — p_new of an even iteration is pp[1]
-			auto kf = pcg_flush_x_kernel<T>;
-			FI_LAUNCH(kf, grid, kThreads, 0, s, n, x + off, static_cast<const T*>(pp[1] + off), static_cast<const PcgState*>(w.state.data()));
+		const int pending = deferred_x ? static_cast<int>(h.iters % ring) : 0;
+		if (pending > 0) {
+			// the last `pending` iterations (ring positions 0 .. pending-1, whichever way the loop stopped: convergence, the
+			// iteration cap or a breakdown, which parks nothing) left their x update parked; p_j of position i is in dir[i + 1].
+			// Their step lengths are in PcgWork::alpha, on a slab (m = 2) in PcgState::alpha_prev.
+			DirRing<T> d = {};
+			for (int i = 0; i < pending; ++i) { d.p[i] = w.dir[i + 1].data() + off; }
+			const double* parked = dist ? &w.state.data()->alpha_prev : w.alpha.data();
+			auto          kf     = pcg_flush_x_kernel<T>;
+			FI_LAUNCH(kf, grid, kThreads, 0, s, n, x + off, d, parked, pending);
 		}
+		res.x_ring = deferred_x ? ring : 1;
 		FI_CUDA(cudaEventRecord(l1, s));
 		FI_CUDA(cudaEventSynchronize(l1));
 		if (link && trace_enabled() && h.iters >= 8) {
@@ -920,16 +1111,20 @@ void time_kernels(Operator<T>& op, int iterations, int check_every, double* out,
 		return static_cast<double>(ms);
 	};
 	DevBuf<double> dot(1);
-	T*             pp[2] = {w.p.data(), w.p2.data()};
-	bool           fused = false;
+	// the directions as the solve cycles through them: ring position i mod m reads dir[i mod m] and writes the next one
+	const int m     = std::max(2, r.x_ring);
+	T*        p0    = w.dir[0].data();
+	auto      p_old = [&](int i) { return w.dir[i % m].data(); };
+	auto      p_new = [&](int i) { return w.dir[(i + 1) % m].data(); };
+	bool      fused = false;
 	out[1] = timed([&](int i) {
 		const int par = i & 1;
-		fused = stencil_fused_step<T>(op.use_fast, op.g, op.tabs, w.r.data(), op.minv.data(), pp[par], pp[par ^ 1], w.q.data(),
+		fused = stencil_fused_step<T>(op.use_fast, op.g, op.tabs, w.r.data(), op.minv.data(), p_old(i), p_new(i), w.q.data(),
 		                              w.state.data(), par, dot.data(), op.partial.data(), op.ticket.data(), nullptr, s);
 		if (fused) {
-			apply_data_term<T>(op.g, op.data, pp[par ^ 1], w.q.data(), dot.data(), nullptr, s);
+			apply_data_term<T>(op.g, op.data, p_new(i), w.q.data(), dot.data(), nullptr, s);
 		} else {
-			op.apply(w.p.data(), w.q.data(), dot.data(), nullptr, s);
+			op.apply(p0, w.q.data(), dot.data(), nullptr, s);
 		}
 	});
 	// alpha = rho/pq is recomputed from the (frozen) state each launch; a tiny alpha keeps the vectors finite
@@ -937,44 +1132,37 @@ void time_kernels(Operator<T>& op, int iterations, int check_every, double* out,
 	FI_CUDA(cudaMemcpyAsync(w.state.data(), &h, sizeof(h), cudaMemcpyHostToDevice, s));
 	FI_CUDA(cudaStreamSynchronize(s));
 	out[2] = timed([&](int i) {
-		// the fused path alternates an iteration that leaves x alone with one that applies two terms (deferred x update)
+		// the fused path runs m-1 launches that leave x alone and one that applies m terms per ring of m iterations
 		if (!fused) {
 			auto ku = pcg_update_kernel<T, kXClassic>;
-			FI_LAUNCH(ku, vec_grid(n), kThreads, 0, s, n, x.data(), w.r.data(), w.p.data(), static_cast<const T*>(nullptr), w.q.data(), op.minv.data(), w.state.data(), 0,
+			FI_LAUNCH(ku, vec_grid(n), kThreads, 0, s, n, x.data(), w.r.data(), p0, static_cast<const T*>(nullptr), w.q.data(), op.minv.data(), w.state.data(), 0,
 			          w.partial.data(), w.ticket.data(), 0);  // reads rho[0], pq (frozen); writes rho[1], rr, iters
-		} else if ((i & 1) == 0) {
-			auto ku = pcg_update_kernel<T, kXSkip>;
-			FI_LAUNCH(ku, vec_grid(n), kThreads, 0, s, n, x.data(), w.r.data(), w.p2.data(), w.p.data(), w.q.data(), op.minv.data(), w.state.data(), 0,
-			          w.partial.data(), w.ticket.data(), 0);
 		} else {
-			auto ku = pcg_update_kernel<T, kXBoth>;
-			FI_LAUNCH(ku, vec_grid(n), kThreads, 0, s, n, x.data(), w.r.data(), w.p.data(), w.p2.data(), w.q.data(), op.minv.data(), w.state.data(), 0,
-			          w.partial.data(), w.ticket.data(), 0);
+			launch_ring_update<T>(w, m, i % m, vec_grid(n), n, x.data(), op.minv.data(), 0, s);
 		}
 	});
 	out[3] = 0.0;
 	if (!fused) {
 		out[3] = timed([&](int) {
 			auto kd = pcg_direction_kernel<T>;
-			FI_LAUNCH(kd, vec_grid(n), kThreads, 0, s, n, w.r.data(), op.minv.data(), w.p.data(), w.state.data(), 0);
+			FI_LAUNCH(kd, vec_grid(n), kThreads, 0, s, n, w.r.data(), op.minv.data(), p0, w.state.data(), 0);
 		});
 	}
 	out[4] = fused ? 1.0 : 0.0;
-	out[7] = 0.0;
+	out[7] = fused ? m : 1;
 	// the two halves of the apply on their own: the lattice-sized stencil kernel (the dominant kernel of the roofline
 	// figure) and the data-term kernels over the occupied cells
 	out[5] = timed([&](int i) {
 		const int par = i & 1;
 		if (fused) {
-			stencil_fused_step<T>(op.use_fast, op.g, op.tabs, w.r.data(), op.minv.data(), pp[par], pp[par ^ 1], w.q.data(), w.state.data(), par,
+			stencil_fused_step<T>(op.use_fast, op.g, op.tabs, w.r.data(), op.minv.data(), p_old(i), p_new(i), w.q.data(), w.state.data(), par,
 			                      dot.data(), op.partial.data(), op.ticket.data(), nullptr, s);
 		} else {
-			stencil_apply<T>(op.g, op.tabs, w.p.data(), w.q.data(), dot.data(), op.partial.data(), op.ticket.data(), nullptr, op.use_fast, s);
+			stencil_apply<T>(op.g, op.tabs, p0, w.q.data(), dot.data(), op.partial.data(), op.ticket.data(), nullptr, op.use_fast, s);
 		}
 	});
 	out[6] = timed([&](int i) {
-		const int par = i & 1;
-		apply_data_term<T>(op.g, op.data, fused ? pp[par ^ 1] : w.p.data(), w.q.data(), dot.data(), nullptr, s);
+		apply_data_term<T>(op.g, op.data, fused ? p_new(i) : p0, w.q.data(), dot.data(), nullptr, s);
 	});
 	cudaEventDestroy(e0);
 	cudaEventDestroy(e1);

@@ -44,11 +44,18 @@ struct DistHooks
 	}
 };
 
+// Most search directions the fused PCG iteration keeps before it folds their terms into x (solver.cu, choose_x_ring).
+constexpr int kMaxXRing = 8;
+
 template <typename T>
 struct PcgWork
 {
-	DevBuf<T>        r, p, q;
-	DevBuf<T>        p2;  // ping-pong partner of p for the fused direction+stencil kernel
+	DevBuf<T>        r, q;
+	// Search directions.  The fused direction+stencil iteration k reads dir[k mod m] and writes dir[(k+1) mod m] (m = the
+	// x ring of the solve, 2 on slab-sharded lattices: the ping-pong pair dir[0] / dir[1]); the unfused iteration uses dir[0].
+	DevBuf<T>        dir[kMaxXRing];
+	int              dirs = 0;  // dir[0 .. dirs) are allocated (lattice-sized, zeroed when allocated)
+	DevBuf<double>   alpha;     // step lengths of the iterations whose x update is still pending (kMaxXRing - 1)
 	DevBuf<double>   partial;
 	DevBuf<unsigned> ticket;
 	DevBuf<PcgState> state;
@@ -90,6 +97,7 @@ struct PcgResult
 	long long iterations = 0;
 	double    rel_residual = 0, initial_residual = 0, true_residual = 0, solve_ms = 0;
 	double    loop_ms = 0;  // graph launches only (no init, capture or instantiation)
+	int       x_ring = 1;   // iterations per x update: the ring of directions the fused path kept (1: the unfused iteration)
 	bool      converged = false, zero_rhs = false;
 	// The iteration cannot get further in this arithmetic: CG broke down, or the residual recomputed from x stopped
 	// following the recurrence (an fp32 solve at the rounding floor of an ill-conditioned system).  The caller may continue

@@ -418,12 +418,14 @@ FI_API void    fi_kernel_launches_reset(void);
  *   ms[0] `iterations` whole PCG iterations as fi_field_solve runs them (CUDA graph, no convergence stop)
  *   ms[1] the operator-apply kernels alone, back to back: the fused direction+stencil kernel when the solve
  *         uses it, else the stencil kernel (plus the data-term kernels)
- *   ms[2] the update kernel alone (x += a p, r -= a q, r.Mr, r.r)
+ *   ms[2] the update kernel alone (x += a p, r -= a q, r.Mr, r.r); on the fused path in the forms the solve runs, m-1
+ *         launches that leave x alone and one that adds the m pending terms to x per ring of m iterations
  *   ms[3] the direction kernel alone (0 when it is fused into the stencil)
  *   ms[4] 1 if the fused kernel is in use, else 0
  *   ms[5] the lattice-sized stencil kernel of ms[1] alone (the dominant kernel of the roofline figure)
  *   ms[6] the data-term kernels of ms[1] alone (occupied-cell blocks + generic rows)
- * `ms` must hold 8 doubles (ms[7] is reserved, written as 0). */
+ *   ms[7] m: iterations per x update of the solve (FI_B200_X_RING; 1 when the fused kernel is not in use)
+ * `ms` must hold 8 doubles. */
 FI_API int fi_field_time_iterations(fi_field* f, const fi_solve_options* opt, int32_t iterations, double* ms);
 
 #ifdef __cplusplus
