@@ -64,6 +64,22 @@ class fi_cascade_stats(C.Structure):
                 "total_ms": self.total_ms, "cell_iterations": self.cell_iterations, "finest": self.finest.as_dict()}
 
 
+FI_MG_MAX_LEVELS = 20
+FI_MG_CYCLE, FI_MG_OPERATOR, FI_MG_RESTRICT, FI_MG_PROLONG_ADD, FI_MG_SMOOTH, FI_MG_COARSE = range(6)
+
+
+class fi_mg_info(C.Structure):
+    _fields_ = [("levels", C.c_int32), ("sizes", (C.c_int32 * 3) * FI_MG_MAX_LEVELS), ("lmax", C.c_double * FI_MG_MAX_LEVELS),
+                ("nu", C.c_int32), ("nu_coarse", C.c_int32), ("gamma", C.c_int32), ("w_levels", C.c_int32),
+                ("cheb_ratio", C.c_double), ("tail_from", C.c_int32), ("coarsest", C.c_int32)]
+
+    def as_dict(self):
+        L = self.levels
+        return {"levels": L, "sizes": [list(self.sizes[l]) for l in range(L)], "lmax": list(self.lmax[:L]), "nu": self.nu,
+                "nu_coarse": self.nu_coarse, "gamma": self.gamma, "w_levels": self.w_levels, "cheb_ratio": self.cheb_ratio,
+                "tail_from": self.tail_from, "coarsest": self.coarsest}
+
+
 _p = C.POINTER
 _vp, _i32, _i64, _f, _d = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_double
 _pf, _pi32, _pi64, _pd = _p(C.c_float), _p(C.c_int32), _p(C.c_int64), _p(C.c_double)
@@ -119,6 +135,8 @@ SIGNATURES = {
     "fi_kernel_launches": (_i64, []),
     "fi_kernel_launches_reset": (None, []),
     "fi_field_time_iterations": (C.c_int, [_vp, _p(fi_solve_options), _i32, _pd]),
+    "fi_field_mg_info": (C.c_int, [_vp, _p(fi_solve_options), _p(fi_mg_info)]),
+    "fi_field_mg_stage": (C.c_int, [_vp, _p(fi_solve_options), _i32, _i32, _i64, _vp, _vp, _vp]),
 }
 
 _dll = None

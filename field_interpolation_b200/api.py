@@ -210,6 +210,35 @@ class LatticeField:
         return {"iteration_ms": ms[0], "apply_ms": ms[1], "update_ms": ms[2], "direction_ms": ms[3], "fused": bool(ms[4]),
                 "stencil_ms": ms[5], "data_term_ms": ms[6], "x_ring": int(ms[7])}
 
+    # ---- the multigrid preconditioner, stage by stage (fi_field_mg_info / fi_field_mg_stage; for tests) ----------------
+    def mg_info(self, options: Optional[L.fi_solve_options] = None) -> dict:
+        """The hierarchy an FI_PRECOND_MULTIGRID solve with `options` uses: levels, sizes (x y z per level), lmax per
+        smoothed level, nu, nu_coarse, gamma, w_levels, cheb_ratio, tail_from, coarsest."""
+        opt = options if options is not None else solve_options(preconditioner=FI_PRECOND_MULTIGRID)
+        info = L.fi_mg_info()
+        L.check(L.lib().fi_field_mg_info(self._h, C.byref(opt), C.byref(info)))
+        return info.as_dict()
+
+    def mg_stage(self, stage: int, level: int, x, x2=None, options: Optional[L.fi_solve_options] = None) -> np.ndarray:
+        """One stage of the cycle (L.FI_MG_*) on level `level` applied to x: one vector (n,) or a batch (count, n), fp32.
+        x2: the vector PROLONG_ADD adds to / SMOOTH starts from (None: zero), same batch shape as the result."""
+        opt = options if options is not None else solve_options(preconditioner=FI_PRECOND_MULTIGRID)
+        info = self.mg_info(opt)
+        cells = [int(np.prod(s)) for s in info["sizes"]]
+        if not 0 <= level < info["levels"]:
+            raise ValueError(f"level {level} of a {info['levels']}-level hierarchy")
+        n_in = cells[level + 1] if stage == L.FI_MG_PROLONG_ADD else cells[level]
+        n_out = cells[level + 1] if stage == L.FI_MG_RESTRICT else cells[level]
+        xi = np.ascontiguousarray(x, np.float32)
+        single = xi.ndim == 1
+        xi = xi.reshape(-1, n_in)
+        count = xi.shape[0]
+        x2i = None if x2 is None else np.ascontiguousarray(x2, np.float32).reshape(count, n_out)
+        out = np.empty((count, n_out), np.float32)
+        L.check(L.lib().fi_field_mg_stage(self._h, C.byref(opt), int(stage), int(level), count, C.c_void_p(xi.ctypes.data),
+                                          None if x2i is None else C.c_void_p(x2i.ctypes.data), C.c_void_p(out.ctypes.data)))
+        return out[0] if single else out
+
 
 # ---- builders (field_interpolation.hpp:116-173) ------------------------------------------------------
 

@@ -1423,4 +1423,26 @@ int fi_field_time_iterations(fi_field* f, const fi_solve_options* opt, int32_t i
 	});
 }
 
+int fi_field_mg_info(fi_field* f, const fi_solve_options* opt, fi_mg_info* out)
+{
+	return guarded([&] {
+		FI_REQUIRE(f && out, FI_ERR_INVALID, "bad argument");
+		fi_solve_options o;
+		if (opt) { o = *opt; } else { fi_solve_options_default(&o); }
+		mg_info(f->get_mg(o), out);
+	});
+}
+
+int fi_field_mg_stage(fi_field* f, const fi_solve_options* opt, int32_t stage, int32_t level, int64_t count, const float* in, const float* in2, float* out)
+{
+	return guarded([&] {
+		FI_REQUIRE(f != nullptr, FI_ERR_INVALID, "field is null");
+		fi_solve_options o;
+		if (opt) { o = *opt; } else { fi_solve_options_default(&o); }
+		Multigrid& mg = f->get_mg(o);
+		f->get32().use_fast = o.use_fast_stencil;  // the fine level's kernels as an FI_F32 solve with `o` picks them
+		mg_stage(mg, stage, level, count, in, in2, out, f->stream);
+	});
+}
+
 }  // extern "C"

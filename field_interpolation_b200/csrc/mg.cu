@@ -1038,7 +1038,7 @@ std::unique_ptr<Multigrid> build_multigrid(Operator<float>& fine, const ModelAcc
 	// largest eigenvalue of D^-1 A per smoothed level: power iteration
 	{
 		TraceScope tp("power iterations");
-		// v_k = (D^-1 A)^k v_0 without normalising in between (|v| grows by lambda <= ~4 per round: 12 rounds stay far inside
+		// v_k = (D^-1 A)^k v_0 without normalising in between (|v| grows by lambda <= ~8 per round: 20 rounds stay far inside
 		// fp32) — the squared norms of all rounds and levels are read back once, lambda = |v_K| / |v_K-1|.  Normalising every
 		// round cost a kernel over the level and a host synchronisation each (16.6 ms at 512^3, profiles/r2p_trace_time_to_tol_512.txt).
 		const int        K = std::max(2, opt.power_iterations);
@@ -1256,6 +1256,88 @@ bool Multigrid::demote_to_v_cycle()
 		exec = nullptr;
 	}
 	return true;
+}
+
+// ---- test hook: the hierarchy and one stage of its cycle ---------------------------------------------------------------
+void mg_info(const Multigrid& mg, fi_mg_info* out)
+{
+	const int L = static_cast<int>(mg.levels.size());
+	FI_REQUIRE(L <= FI_MG_MAX_LEVELS, FI_ERR_RANGE, "multigrid: more levels than fi_mg_info holds");
+	std::memset(out, 0, sizeof(*out));
+	out->levels = L;
+	for (int l = 0; l < L; ++l) {
+		const Multigrid::Level& lv = *mg.levels[l];
+		for (int d = 0; d < kMaxDim; ++d) { out->sizes[l][d] = d < lv.g.ndim ? lv.g.size[d] : 1; }
+		out->lmax[l] = l + 1 < L ? lv.lmax : 0.0;
+	}
+	out->nu         = mg.opt.nu;
+	out->nu_coarse  = mg.opt.nu_coarse;
+	out->gamma      = mg.opt.gamma;
+	out->w_levels   = mg.opt.w_levels;
+	out->cheb_ratio = mg.opt.cheb_ratio;
+	out->tail_from  = mg.tail_from;
+	out->coarsest   = mg.nc;
+}
+
+void mg_stage(Multigrid& mg, int stage, int level, int64_t count, const float* in, const float* in2, float* out, cudaStream_t s)
+{
+	const int L = static_cast<int>(mg.levels.size());
+	FI_REQUIRE(level >= 0 && level < L, FI_ERR_INVALID, "mg_stage: no such level");
+	FI_REQUIRE(count >= 0 && (count == 0 || (in != nullptr && out != nullptr)), FI_ERR_INVALID, "mg_stage: in / out is null");
+	Multigrid::Level& lv = *mg.levels[level];
+	const bool        coarser = level + 1 < L;
+	const int64_t     n = lv.g.N, nc = coarser ? mg.levels[level + 1]->g.N : 0;
+	int64_t           n_in = n, n_out = n;
+	bool              takes_in2 = false;
+	switch (stage) {
+	case FI_MG_CYCLE: FI_REQUIRE(level == 0, FI_ERR_INVALID, "mg_stage: the cycle starts at level 0"); break;
+	case FI_MG_OPERATOR: break;
+	case FI_MG_RESTRICT:
+		FI_REQUIRE(coarser, FI_ERR_INVALID, "mg_stage: the coarsest level restricts nowhere");
+		n_out = nc;
+		break;
+	case FI_MG_PROLONG_ADD:
+		FI_REQUIRE(coarser, FI_ERR_INVALID, "mg_stage: nothing prolongs into the coarsest level");
+		n_in      = nc;
+		takes_in2 = true;
+		break;
+	case FI_MG_SMOOTH:
+		FI_REQUIRE(coarser, FI_ERR_INVALID, "mg_stage: the coarsest level is solved, not smoothed");
+		takes_in2 = true;
+		break;
+	case FI_MG_COARSE: FI_REQUIRE(level == L - 1, FI_ERR_INVALID, "mg_stage: the dense solve is on the coarsest level"); break;
+	default: throw Error{FI_ERR_INVALID, "mg_stage: unknown stage"};
+	}
+	if (stage == FI_MG_CYCLE && mg.exec) {  // capture afresh: the caller may have changed the fine operator's kernel choice
+		cudaGraphExecDestroy(mg.exec);
+		mg.exec = nullptr;
+	}
+	DevBuf<float> din(static_cast<size_t>(n_in)), dout(static_cast<size_t>(n_out));
+	const int     nu = (level + mg.base_level > 0 && mg.opt.nu_coarse > 0) ? mg.opt.nu_coarse : mg.opt.nu;
+	for (int64_t k = 0; k < count; ++k) {
+		FI_CUDA(cudaMemcpyAsync(din.data(), in + k * n_in, n_in * sizeof(float), cudaMemcpyHostToDevice, s));
+		if (takes_in2) {
+			if (in2) {
+				FI_CUDA(cudaMemcpyAsync(dout.data(), in2 + k * n_out, n_out * sizeof(float), cudaMemcpyHostToDevice, s));
+			} else {
+				dout.zero(s);
+			}
+		}
+		switch (stage) {
+		case FI_MG_CYCLE: mg.vcycle(din.data(), dout.data(), s); break;
+		case FI_MG_OPERATOR: lv.op->apply(din.data(), dout.data(), nullptr, nullptr, s); break;
+		case FI_MG_RESTRICT: {
+			const Xfer& x = lv.to_coarser;
+			FI_LAUNCH(restrict_kernel, dim3(div_up(x.nc[0], 128), div_up(x.nc[1], kXferRows), x.nc[2]), 128, 0, s, x, din.data(), dout.data());
+			break;
+		}
+		case FI_MG_PROLONG_ADD: launch_prolong_add(lv.to_coarser, lv.to_coarser.nf[2], din.data(), dout.data(), s); break;
+		case FI_MG_SMOOTH: smooth(lv, mg.opt, nu, din.data(), dout.data(), in2 == nullptr, s); break;
+		case FI_MG_COARSE: FI_LAUNCH(dense_matvec_kernel, mg.nc, 128, 0, s, mg.nc, mg.coarse_inv.data(), din.data(), dout.data()); break;
+		}
+		FI_CUDA(cudaMemcpyAsync(out + k * n_out, dout.data(), n_out * sizeof(float), cudaMemcpyDeviceToHost, s));
+		FI_CUDA(cudaStreamSynchronize(s));
+	}
 }
 
 // ---- the V-cycle with z-slab sharded fine levels ------------------------------------------------------------------------

@@ -164,7 +164,10 @@ struct MgOptions
 	                                 // W-cycle would visit them 2^level times for no gain but launch latency
 	double cheb_ratio       = 12.0;  // the smoother targets the eigenvalues of D^-1 A in [lambda_max / ratio, lambda_max]
 	int    coarsest_cells   = 600;   // coarsen until a level has at most this many cells (dense solve there, inverse computed on the device)
-	int    power_iterations = 12;    // for lambda_max, per level, at setup
+	int    power_iterations = 20;    // for lambda_max, per level, at setup.  The top of the spectrum of D^-1 A is dense, so the estimate
+	                                 // creeps up slowly: after 12 rounds it was 0.877 lambda_max on a 48 x 20 level, and 1.1 times that is
+	                                 // below lambda_max (the smoother then amplifies the top modes); 20 rounds reach >= 0.93 on every level
+	                                 // of tests/test_gpu_multigrid_operator.py
 	int    tail_cells       = 0;     // > 0: coarse levels with at most this many nodes are walked by ONE kernel (mg_tail_kernel) instead of
 	                                 // three launches per smoothing step (FI_B200_MG_TAIL_CELLS).  Off by default: measured slower — one SM
 	                                 // retires the data term's reductions at 1.3 cycles per lane, 283 us per visit of a 16^3 level against
@@ -236,6 +239,11 @@ struct Multigrid
 // level's operator is the one the single-GPU hierarchy would have.
 std::unique_ptr<Multigrid> build_multigrid(Operator<float>& fine, const ModelAccum& model, const PointStore& pts, const MgOptions& opt, cudaStream_t s,
                                            const int* root_size = nullptr, int fine_level = 0);
+
+// The hierarchy's shape and parameters (fi_field_mg_info), and one stage of its cycle applied to `count` host vectors
+// (fi_field_mg_stage: stage FI_MG_*, the kernels vcycle() runs, on scratch vectors of its own).  For tests.
+void mg_info(const Multigrid& mg, fi_mg_info* out);
+void mg_stage(Multigrid& mg, int stage, int level, int64_t count, const float* in, const float* in2, float* out, cudaStream_t s);
 
 // ---- mg.cu: the same V-cycle with the finest levels z-slab sharded over the ranks of a communicator -------------
 // Levels 0 .. nd-1 are sharded (each rank smooths its slab; halo planes of the smoothed vector are exchanged before

@@ -30,7 +30,8 @@ extern "C" {
 /* 5: + fi_sample_field (additions only) */
 /* 6: + fi_field_error_map (additions only) */
 /* 7: + fi_nearest_point_distance, fi_field_add_border_distance (additions only) */
-#define FI_B200_ABI_VERSION 7
+/* 8: + fi_field_mg_info, fi_field_mg_stage (additions only) */
+#define FI_B200_ABI_VERSION 8
 
 #if defined(__GNUC__)
 #define FI_API __attribute__((visibility("default")))
@@ -427,6 +428,37 @@ FI_API void    fi_kernel_launches_reset(void);
  *   ms[7] m: iterations per x update of the solve (FI_B200_X_RING; 1 when the fused kernel is not in use)
  * `ms` must hold 8 doubles. */
 FI_API int fi_field_time_iterations(fi_field* f, const fi_solve_options* opt, int32_t iterations, double* ms);
+
+/* ---- multigrid preconditioner, stage by stage (for tests) ------------------------------------------------------ */
+/* The hierarchy FI_PRECOND_MULTIGRID solves with `opt` use (built on first use, the same object the solve then reuses).
+ * Level 0 is the field's own lattice; unused axes have size 1. */
+#define FI_MG_MAX_LEVELS 20
+typedef struct fi_mg_info {
+	int32_t levels;
+	int32_t sizes[FI_MG_MAX_LEVELS][3];
+	double  lmax[FI_MG_MAX_LEVELS];  /* Chebyshev upper bound on the eigenvalues of D^-1 A_l, levels 0 .. levels-2; 0 for the coarsest */
+	int32_t nu;                      /* Chebyshev steps on level 0 (and on every level when nu_coarse == 0) */
+	int32_t nu_coarse;               /* ... on levels >= 1; 0: nu */
+	int32_t gamma;                   /* 1: V-cycle; 2: W-cycle on the coarse problems of levels 1 .. w_levels */
+	int32_t w_levels;
+	double  cheb_ratio;              /* smoothed interval [lmax / cheb_ratio, lmax] */
+	int32_t tail_from;               /* first level walked by the single-kernel tail of the cycle; 0: none */
+	int32_t coarsest;                /* nodes of the coarsest level (dense solve) */
+} fi_mg_info;
+FI_API int fi_field_mg_info(fi_field* f, const fi_solve_options* opt, fi_mg_info* out);
+
+enum {
+	FI_MG_CYCLE       = 0, /* out = B in: one application of the preconditioner (level 0) */
+	FI_MG_OPERATOR    = 1, /* out = A_l in */
+	FI_MG_RESTRICT    = 2, /* out (level l + 1) = P_l^T in (level l) */
+	FI_MG_PROLONG_ADD = 3, /* out (level l) = in2 + P_l in (in: level l + 1; in2 NULL: zero) */
+	FI_MG_SMOOTH      = 4, /* out = e after the cycle's Chebyshev steps of level l on A_l e = in, from e = in2 (NULL: from zero) */
+	FI_MG_COARSE      = 5  /* out = A_L^-1 in with the stored dense inverse (level L = levels - 1) */
+};
+/* Applies one stage of the cycle to `count` host vectors, stored one after the other in fp32 (in / in2 / out: count
+ * vectors of the sizes above).  Runs the kernels the cycle runs, on scratch vectors of its own. */
+FI_API int fi_field_mg_stage(fi_field* f, const fi_solve_options* opt, int32_t stage, int32_t level, int64_t count, const float* in,
+                             const float* in2, float* out);
 
 #ifdef __cplusplus
 }
