@@ -80,6 +80,31 @@ class fi_mg_info(C.Structure):
                 "tail_from": self.tail_from, "coarsest": self.coarsest}
 
 
+FI_PCG_MAX_RING = 8
+FI_PCG_INIT, FI_PCG_STENCIL, FI_PCG_DATA, FI_PCG_UPDATE, FI_PCG_FLUSH, FI_PCG_UNFUSED = range(6)
+FI_PCG_V_X, FI_PCG_V_R, FI_PCG_V_Q, FI_PCG_V_B, FI_PCG_V_DIR = range(5)
+FI_PCG_KERNEL_NONE, FI_PCG_KERNEL_TMA_3D, FI_PCG_KERNEL_TILED_3D, FI_PCG_KERNEL_TMA_2D = range(4)
+FI_PCG_DATA_CELLS, FI_PCG_DATA_NODES, FI_PCG_DATA_SPLIT, FI_PCG_DATA_ROWS = 1, 2, 4, 8
+
+
+class fi_pcg_state(C.Structure):
+    _fields_ = [("rho", C.c_double * 2), ("pq", C.c_double), ("rr", C.c_double), ("bb", C.c_double), ("tol2bb", C.c_double),
+                ("rr0", C.c_double), ("done", C.c_int32), ("breakdown", C.c_int32), ("iters", C.c_int64), ("max_iters", C.c_int64),
+                ("alpha", C.c_double * (FI_PCG_MAX_RING - 1))]
+
+    def as_dict(self):
+        d = {n: getattr(self, n) for n, _ in self._fields_}
+        d["rho"], d["alpha"] = list(self.rho), list(self.alpha)
+        return d
+
+
+class fi_pcg_report(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("stencil", "radius", "gs", "tile_rows", "z_chunks", "data_term")]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
+
+
 _p = C.POINTER
 _vp, _i32, _i64, _f, _d = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_double
 _pf, _pi32, _pi64, _pd = _p(C.c_float), _p(C.c_int32), _p(C.c_int64), _p(C.c_double)
@@ -137,6 +162,8 @@ SIGNATURES = {
     "fi_field_time_iterations": (C.c_int, [_vp, _p(fi_solve_options), _i32, _pd]),
     "fi_field_mg_info": (C.c_int, [_vp, _p(fi_solve_options), _p(fi_mg_info)]),
     "fi_field_mg_stage": (C.c_int, [_vp, _p(fi_solve_options), _i32, _i32, _i64, _vp, _vp, _vp]),
+    "fi_field_pcg_stage": (C.c_int, [_vp, _p(fi_solve_options), _i32, _i32, _i32, _i32, _i32, _i32, _p(_vp), _p(fi_pcg_state),
+                                     _p(fi_pcg_report)]),
 }
 
 _dll = None

@@ -239,6 +239,52 @@ class LatticeField:
                                           None if x2i is None else C.c_void_p(x2i.ctypes.data), C.c_void_p(out.ctypes.data)))
         return out[0] if single else out
 
+    # ---- the Jacobi-PCG iteration, stage by stage (fi_field_pcg_stage; for tests) ---------------------------------------
+    def pcg_stage(self, stage: int, vectors: dict, state: dict, par: int = 0, pos: int = 0, ring: int = 2, count: int = 0,
+                  options: Optional[L.fi_solve_options] = None):
+        """One stage (L.FI_PCG_*) of the iteration fi_field_solve runs with `options` (precision FI_F32 / FI_F64,
+        use_fast_stencil).  vectors: {"x", "r", "q", "b", "dir": [dir[0], ...]} of N elements each, numpy arrays of the
+        precision's dtype or torch CUDA tensors (all of one kind); missing ones enter as zeros.  state: the fields of
+        fi_pcg_state (missing ones 0).  Returns (vectors after the stage, in new numpy arrays or the same tensors updated in
+        place; state dict; report dict)."""
+        opt = options if options is not None else solve_options(FI_F64)
+        dt = np.float64 if opt.precision == FI_F64 else np.float32
+        n = self.num_unknowns
+        names = ["x", "r", "q", "b"]
+        given = [vectors.get(k) for k in names] + list(vectors.get("dir", []))
+        if len(given) > L.FI_PCG_V_DIR + ring:
+            raise ValueError(f"more directions than a ring of {ring}")
+        given += [None] * (L.FI_PCG_V_DIR + ring - len(given))
+        device = any(_is_device(a) for a in given if a is not None)
+        bufs = []
+        for a in given:
+            if a is None:
+                bufs.append(None)
+            elif device:
+                import torch
+                assert _is_device(a) and a.is_contiguous() and a.numel() == n
+                assert a.dtype == (torch.float64 if dt is np.float64 else torch.float32)
+                bufs.append(a)
+            else:
+                h = np.array(a, dtype=dt, copy=True).reshape(-1)
+                assert h.size == n
+                bufs.append(h)
+        ptrs = (C.c_void_p * len(bufs))(*[None if b is None else (b.data_ptr() if device else b.ctypes.data) for b in bufs])
+        st = L.fi_pcg_state()
+        for k, v in state.items():
+            if k in ("rho", "alpha"):
+                arr = getattr(st, k)
+                for i, e in enumerate(v):
+                    arr[i] = e
+            else:
+                setattr(st, k, v)
+        rep = L.fi_pcg_report()
+        L.check(L.lib().fi_field_pcg_stage(self._h, C.byref(opt), int(stage), int(par), int(pos), int(ring), int(count),
+                                           FI_DEVICE if device else FI_HOST, ptrs, C.byref(st), C.byref(rep)))
+        out = {k: b for k, b in zip(names, bufs[:4]) if b is not None}
+        out["dir"] = bufs[4:]
+        return out, st.as_dict(), rep.as_dict()
+
 
 # ---- builders (field_interpolation.hpp:116-173) ------------------------------------------------------
 

@@ -16,6 +16,7 @@
 namespace fi {
 
 int64_t                   g_launches = 0;
+LaunchNote                g_note;
 static thread_local std::string t_last_error;
 
 void set_last_error(const std::string& s) { t_last_error = s; }
@@ -1442,6 +1443,26 @@ int fi_field_mg_stage(fi_field* f, const fi_solve_options* opt, int32_t stage, i
 		Multigrid& mg = f->get_mg(o);
 		f->get32().use_fast = o.use_fast_stencil;  // the fine level's kernels as an FI_F32 solve with `o` picks them
 		mg_stage(mg, stage, level, count, in, in2, out, f->stream);
+	});
+}
+
+int fi_field_pcg_stage(fi_field* f, const fi_solve_options* opt, int32_t stage, int32_t par, int32_t pos, int32_t ring, int32_t count, int32_t loc,
+                       void* const* vectors, fi_pcg_state* state, fi_pcg_report* report)
+{
+	return guarded([&] {
+		FI_REQUIRE(f != nullptr, FI_ERR_INVALID, "field is null");
+		fi_solve_options o;
+		if (opt) { o = *opt; } else { fi_solve_options_default(&o); }
+		if (o.precision == FI_F64) {
+			Operator<double>& op = f->get64();
+			op.use_fast = o.use_fast_stencil;
+			pcg_stage<double>(op, stage, par, pos, ring, count, loc, vectors, o.tolerance, o.max_iterations, state, report, f->stream);
+		} else {
+			FI_REQUIRE(o.precision == FI_F32, FI_ERR_INVALID, "precision must be FI_F32 or FI_F64");
+			Operator<float>& op = f->get32();
+			op.use_fast = o.use_fast_stencil;
+			pcg_stage<float>(op, stage, par, pos, ring, count, loc, vectors, o.tolerance, o.max_iterations, state, report, f->stream);
+		}
 	});
 }
 

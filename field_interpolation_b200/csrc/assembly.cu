@@ -1309,11 +1309,13 @@ bool apply_data_term(const Geom& g, const DataTerm<T>& dt, const T* p, T* q, dou
 					auto kern = apply_nodes_kernel<T, decltype(dim)::value>;
 					FI_LAUNCH(kern, div_up(dt.nnode, kThreads), kThreads, 0, s, g, dt.nnode, dt.node_index.data(), dt.node_coef.data(), p, q, partial, ticket,
 					          d_dot_accum, d_done);
+					g_note.data_term |= FI_PCG_DATA_NODES;
 				}
 			} else if (data_term_kernel() == kDataSplit) {
 				auto kern = apply_blocks_split_kernel<T, decltype(dim)::value>;
 				FI_LAUNCH(kern, gb, kThreads, 0, s, g, dt.nocc, dt.cell_base.data(), dt.cell_mask.data(), dt.blocks.data(), p, q, partial, ticket,
 				          d_dot_accum, d_done);
+				g_note.data_term |= FI_PCG_DATA_SPLIT;
 			} else {
 				// the last block to finish may publish the rank's p.Ap itself (only when nothing else adds to it afterwards)
 				const bool do_pub = pub != nullptr && d_dot_accum != nullptr && gr == 0;
@@ -1321,6 +1323,7 @@ bool apply_data_term(const Geom& g, const DataTerm<T>& dt, const T* p, T* q, dou
 				FI_LAUNCH(kern, gb, kThreads, 0, s, g, dt.nocc, dt.cell_base.data(), dt.cell_mask.data(), dt.blocks.data(), p, q, partial, ticket,
 				          d_dot_accum, d_done, static_cast<const uint64_t*>(nullptr), do_pub ? *pub : PeerPublish(), do_pub ? 1 : 0);
 				published = do_pub;
+				g_note.data_term |= FI_PCG_DATA_CELLS;
 			}
 		});
 	}
@@ -1332,6 +1335,7 @@ bool apply_data_term(const Geom& g, const DataTerm<T>& dt, const T* p, T* q, dou
 		auto kern = apply_rows_kernel<T>;
 		FI_LAUNCH(kern, gr, kThreads, 0, s, dt.nrows, dt.row_ptr.data(), dt.col.data(), dt.val.data(), p, q,
 		          partial + gp + 1, ticket + 1, d_dot_accum, d_done);
+		g_note.data_term |= FI_PCG_DATA_ROWS;
 	}
 	return published;
 }

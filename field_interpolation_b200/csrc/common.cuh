@@ -43,6 +43,22 @@ void set_last_error(const std::string& s);
 extern int64_t g_launches;
 inline void count_launch(int n = 1) { g_launches += n; }
 
+// What the last stencil and data-term launches on the host were (FI_PCG_KERNEL_* / FI_PCG_DATA_*, fi_field_pcg_stage
+// reports it): the tests that compare one kernel with a reference assert the instantiation they mean to cover.
+struct LaunchNote
+{
+	int stencil = 0, radius = 0, gs = 0, tile_rows = 0, z_chunks = 0, data_term = 0;
+};
+extern LaunchNote g_note;
+inline void note_stencil(int kind, int radius, bool gs, int tile_rows, int z_chunks)
+{
+	g_note.stencil   = kind;
+	g_note.radius    = radius;
+	g_note.gs        = gs ? 1 : 0;
+	g_note.tile_rows = tile_rows;
+	g_note.z_chunks  = z_chunks;
+}
+
 #ifndef FI_LAUNCH  // tests/emu/cuda_emu.hpp (the CPU functional emulator of the build container) supplies its own
 #define FI_LAUNCH(kernel, grid, block, smem, stream, ...)                 \
 	do {                                                                  \

@@ -667,6 +667,40 @@ void ensure_work(Operator<T>& op, cudaStream_t s)
 	}
 }
 
+// r = b - q (q = A x, or a zero guess), p_0 = dir[0] = M r and the initial state (on a slab: this rank's partial sums)
+template <typename T>
+void launch_init(Operator<T>& op, const T* rhs, bool zero_guess, T* r_vec, double tol, long long max_iter, int grid, cudaStream_t s)
+{
+	PcgWork<T>&   w   = op.work;
+	const int64_t off = op.g.own_offset(), n = op.g.own_cells();
+	auto kern = pcg_init_kernel<T>;
+	FI_LAUNCH(kern, grid, kThreads, 0, s, n, rhs + off, zero_guess ? static_cast<const T*>(nullptr) : w.q.data() + off, op.minv.data() + off, r_vec + off,
+	          w.dir[0].data() + off, w.state.data(), tol, max_iter, w.partial.data(), w.ticket.data(), op.dist ? 1 : 0);
+}
+
+// The unfused iteration after its operator application q = A dir[0]: x += a p, r -= a q, then p = M r + b p in dir[0]
+template <typename T>
+void launch_unfused_update(PcgWork<T>& w, const T* minv, int grid, int64_t n, T* x, int par, cudaStream_t s)
+{
+	T* const p = w.dir[0].data();
+	auto ku = pcg_update_kernel<T, kXClassic>;
+	FI_LAUNCH(ku, grid, kThreads, 0, s, n, x, w.r.data(), p, static_cast<const T*>(nullptr), w.q.data(), minv, w.state.data(), par, w.partial.data(),
+	          w.ticket.data(), 0);
+	auto kd = pcg_direction_kernel<T>;
+	FI_LAUNCH(kd, grid, kThreads, 0, s, n, w.r.data(), minv, p, w.state.data(), par);
+}
+
+// The x update of the `pending` iterations (ring positions 0 .. pending-1) still parked when the loop stopped: p_j of position
+// i is in dir[i + 1], its step length in parked[i]
+template <typename T>
+void launch_pending_flush(PcgWork<T>& w, int pending, int grid, int64_t n, int64_t off, T* x, const double* parked, cudaStream_t s)
+{
+	DirRing<T> d = {};
+	for (int i = 0; i < pending; ++i) { d.p[i] = w.dir[i + 1].data() + off; }
+	auto kf = pcg_flush_x_kernel<T>;
+	FI_LAUNCH(kf, grid, kThreads, 0, s, n, x + off, d, parked, pending);
+}
+
 }  // namespace
 
 void convert(const float* src, double* dst, int64_t n, cudaStream_t s)
@@ -785,9 +819,7 @@ PcgResult pcg_solve(Operator<T>& op, const T* b, T* x, double tol, long long max
 	}
 	{
 		// p goes to dir[0]: the p_old of iteration 0 (read times beta = 0)
-		auto kern = pcg_init_kernel<T>;
-		FI_LAUNCH(kern, grid, kThreads, 0, s, n, rhs + off, zero_guess ? static_cast<const T*>(nullptr) : w.q.data() + off, op.minv.data() + off, r_vec + off, w.dir[0].data() + off,
-		          w.state.data(), tol, max_iter, w.partial.data(), w.ticket.data(), dist ? 1 : 0);
+		launch_init<T>(op, rhs, zero_guess, r_vec, tol, max_iter, grid, s);
 		if (dist) {
 			dist->allreduce(w.state.data()->part, 3, s);
 			FI_LAUNCH(pcg_init_finish_kernel, 1, 1, 0, s, w.state.data(), tol, max_iter);
@@ -867,13 +899,8 @@ PcgResult pcg_solve(Operator<T>& op, const T* b, T* x, double tol, long long max
 					}
 				} else {
 					FI_REQUIRE(dist == nullptr, FI_ERR_UNSUPPORTED, "a slab-sharded solve needs the fused 3D stencil kernel");
-					T* const p = w.dir[0].data();
-					op.apply(p, w.q.data(), d_pq, d_done, s);
-					auto ku = pcg_update_kernel<T, kXClassic>;
-					FI_LAUNCH(ku, grid, kThreads, 0, s, n, x, w.r.data(), p, static_cast<const T*>(nullptr), w.q.data(), op.minv.data(), w.state.data(), par,
-					          w.partial.data(), w.ticket.data(), 0);
-					auto kd = pcg_direction_kernel<T>;
-					FI_LAUNCH(kd, grid, kThreads, 0, s, n, w.r.data(), op.minv.data(), p, w.state.data(), par);
+					op.apply(w.dir[0].data(), w.q.data(), d_pq, d_done, s);
+					launch_unfused_update<T>(w, op.minv.data(), grid, n, x, par, s);
 				}
 			}
 		};
@@ -928,11 +955,7 @@ PcgResult pcg_solve(Operator<T>& op, const T* b, T* x, double tol, long long max
 			// the last `pending` iterations (ring positions 0 .. pending-1, whichever way the loop stopped: convergence, the
 			// iteration cap or a breakdown, which parks nothing) left their x update parked; p_j of position i is in dir[i + 1].
 			// Their step lengths are in PcgWork::alpha, on a slab (m = 2) in PcgState::alpha_prev.
-			DirRing<T> d = {};
-			for (int i = 0; i < pending; ++i) { d.p[i] = w.dir[i + 1].data() + off; }
-			const double* parked = dist ? &w.state.data()->alpha_prev : w.alpha.data();
-			auto          kf     = pcg_flush_x_kernel<T>;
-			FI_LAUNCH(kf, grid, kThreads, 0, s, n, x + off, d, parked, pending);
+			launch_pending_flush<T>(w, pending, grid, n, off, x, dist ? &w.state.data()->alpha_prev : w.alpha.data(), s);
 		}
 		res.x_ring = deferred_x ? ring : 1;
 		FI_CUDA(cudaEventRecord(l1, s));
@@ -1168,6 +1191,106 @@ void time_kernels(Operator<T>& op, int iterations, int check_every, double* out,
 	cudaEventDestroy(e1);
 }
 
+// fi_field_pcg_stage: one stage of the iteration on the solve's own work buffers, through the launch helpers the solve
+// calls, with the caller's vectors copied in and out around it.
+template <typename T>
+void pcg_stage(Operator<T>& op, int stage, int par, int pos, int ring, int count, int loc, void* const* vecs, double tol, long long max_iters,
+               fi_pcg_state* state, fi_pcg_report* report, cudaStream_t s)
+{
+	FI_REQUIRE(vecs != nullptr && state != nullptr, FI_ERR_INVALID, "pcg_stage: vectors / state is null");
+	FI_REQUIRE(loc == FI_HOST || loc == FI_DEVICE, FI_ERR_INVALID, "pcg_stage: unknown loc");
+	FI_REQUIRE(ring == 2 || ring == 4 || ring == 8, FI_ERR_INVALID, "pcg_stage: ring must be 2, 4 or 8");
+	FI_REQUIRE(par == 0 || par == 1, FI_ERR_INVALID, "pcg_stage: par must be 0 or 1");
+	FI_REQUIRE(pos >= 0 && pos < ring, FI_ERR_INVALID, "pcg_stage: pos outside the ring");
+	FI_REQUIRE(stage != FI_PCG_FLUSH || (count >= 1 && count < ring), FI_ERR_INVALID, "pcg_stage: flush count outside 1 .. ring - 1");
+	FI_REQUIRE(stage >= FI_PCG_INIT && stage <= FI_PCG_UNFUSED, FI_ERR_INVALID, "pcg_stage: unknown stage");
+	FI_REQUIRE(op.dist == nullptr && !op.g.sharded() && !op.g.tile, FI_ERR_UNSUPPORTED, "pcg_stage: unsharded lattices only");
+	ensure_work(op, s);
+	PcgWork<T>&   w = op.work;
+	const int64_t n = op.g.N;
+	ensure_ring(w, static_cast<size_t>(n), ring, s);
+	DevBuf<T> x(n), b(n);
+	T* slot[FI_PCG_V_DIR + kMaxXRing] = {x.data(), w.r.data(), w.q.data(), b.data()};
+	for (int j = 0; j < ring; ++j) { slot[FI_PCG_V_DIR + j] = w.dir[j].data(); }
+	const int nslots = FI_PCG_V_DIR + ring;
+	const cudaMemcpyKind in = loc == FI_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+	const cudaMemcpyKind out = loc == FI_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+	for (int k = 0; k < nslots; ++k) {
+		if (vecs[k]) {
+			FI_CUDA(cudaMemcpyAsync(slot[k], vecs[k], n * sizeof(T), in, s));
+		} else {
+			FI_CUDA(cudaMemsetAsync(slot[k], 0, n * sizeof(T), s));
+		}
+	}
+	PcgState h;
+	std::memset(&h, 0, sizeof(h));
+	h.rho[0] = state->rho[0];
+	h.rho[1] = state->rho[1];
+	h.pq = state->pq;
+	h.rr = state->rr;
+	h.bb = state->bb;
+	h.tol2bb = state->tol2bb;
+	h.rr0 = state->rr0;
+	h.done = state->done;
+	h.breakdown = state->breakdown;
+	h.iters = state->iters;
+	h.max_iters = state->max_iters;
+	FI_CUDA(cudaMemcpyAsync(w.state.data(), &h, sizeof(h), cudaMemcpyHostToDevice, s));
+	FI_CUDA(cudaMemcpyAsync(w.alpha.data(), state->alpha, sizeof(state->alpha), cudaMemcpyHostToDevice, s));
+	FI_CUDA(cudaStreamSynchronize(s));
+
+	g_note = LaunchNote();
+	const int  grid   = vec_grid(n);
+	const int* d_done = &w.state.data()->done;
+	double*    d_pq   = &w.state.data()->pq;
+	T* const   p_old  = w.dir[pos].data();
+	T* const   p_new  = w.dir[(pos + 1) % ring].data();
+	switch (stage) {
+	case FI_PCG_INIT: {
+		const bool zero_guess = vecs[FI_PCG_V_X] == nullptr;
+		if (!zero_guess) { op.apply(x.data(), w.q.data(), nullptr, nullptr, s); }
+		launch_init<T>(op, vecs[FI_PCG_V_B] ? b.data() : op.atb.data(), zero_guess, w.r.data(), tol, max_iters, grid, s);
+		break;
+	}
+	case FI_PCG_STENCIL:
+		stencil_fused_step<T>(op.use_fast, op.g, op.tabs, w.r.data(), op.minv.data(), p_old, p_new, w.q.data(), w.state.data(), par, d_pq,
+		                      op.partial.data(), op.ticket.data(), d_done, s);
+		break;
+	case FI_PCG_DATA: apply_data_term<T>(op.g, op.data, p_new, w.q.data(), d_pq, d_done, s); break;
+	case FI_PCG_UPDATE: launch_ring_update<T>(w, ring, pos, grid, n, x.data(), op.minv.data(), par, s); break;
+	case FI_PCG_FLUSH: launch_pending_flush<T>(w, count, grid, n, 0, x.data(), w.alpha.data(), s); break;
+	case FI_PCG_UNFUSED: launch_unfused_update<T>(w, op.minv.data(), grid, n, x.data(), par, s); break;
+	}
+
+	for (int k = 0; k < nslots; ++k) {
+		if (vecs[k]) { FI_CUDA(cudaMemcpyAsync(vecs[k], slot[k], n * sizeof(T), out, s)); }
+	}
+	FI_CUDA(cudaMemcpyAsync(&h, w.state.data(), sizeof(h), cudaMemcpyDeviceToHost, s));
+	FI_CUDA(cudaMemcpyAsync(state->alpha, w.alpha.data(), sizeof(state->alpha), cudaMemcpyDeviceToHost, s));
+	FI_CUDA(cudaStreamSynchronize(s));
+	state->rho[0] = h.rho[0];
+	state->rho[1] = h.rho[1];
+	state->pq = h.pq;
+	state->rr = h.rr;
+	state->bb = h.bb;
+	state->tol2bb = h.tol2bb;
+	state->rr0 = h.rr0;
+	state->done = h.done;
+	state->breakdown = h.breakdown;
+	state->iters = h.iters;
+	state->max_iters = h.max_iters;
+	if (report) {
+		report->stencil   = g_note.stencil;
+		report->radius    = g_note.radius;
+		report->gs        = g_note.gs;
+		report->tile_rows = g_note.tile_rows;
+		report->z_chunks  = g_note.z_chunks;
+		report->data_term = g_note.data_term;
+	}
+}
+
+template void pcg_stage<float>(Operator<float>&, int, int, int, int, int, int, void* const*, double, long long, fi_pcg_state*, fi_pcg_report*, cudaStream_t);
+template void pcg_stage<double>(Operator<double>&, int, int, int, int, int, int, void* const*, double, long long, fi_pcg_state*, fi_pcg_report*, cudaStream_t);
 template void time_kernels<float>(Operator<float>&, int, int, double*, cudaStream_t);
 template void time_kernels<double>(Operator<double>&, int, int, double*, cudaStream_t);
 template std::unique_ptr<Operator<float>> build_operator<float>(const Geom&, const ModelAccum&, const PointStore&, const HostRows&, cudaStream_t);

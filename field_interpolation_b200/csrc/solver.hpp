@@ -313,6 +313,11 @@ void jacobi_sweeps(Operator<T>& op, T* x, int iterations, T weight, cudaStream_t
 template <typename T>
 void time_kernels(Operator<T>& op, int iterations, int check_every, double* out, cudaStream_t s);
 
+// One stage of the unsharded Jacobi-PCG iteration (fi_field_pcg_stage, include/fi_b200.h).  For tests.
+template <typename T>
+void pcg_stage(Operator<T>& op, int stage, int par, int pos, int ring, int count, int loc, void* const* vecs, double tol, long long max_iters,
+               fi_pcg_state* state, fi_pcg_report* report, cudaStream_t s);
+
 // r = b - A x (device), returns |r|^2 and |b|^2.
 template <typename T>
 void residual(Operator<T>& op, const T* b, const T* x, T* r, double* rr, double* bb, cudaStream_t s);

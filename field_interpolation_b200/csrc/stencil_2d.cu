@@ -276,6 +276,7 @@ void launch_2d(const Geom& g, const StencilTables& t, const T* a, const T* b, co
 	}
 	FI_LAUNCH(kern, grid, 256, smem, s, ma, mb, mc, g.size[0], g.size[1], tab, static_cast<T>(t.gs2), q, p_new, st, par, d_dot_out, d_partial, d_ticket, d_done,
 	          epi);
+	note_stencil(FI_PCG_KERNEL_TMA_2D, R, GS, TY, 1);
 }
 
 template <typename T, bool Fused, bool Epi>

@@ -249,6 +249,7 @@ void launch(const Geom& g, const StencilTables& t, const T* p, T* q, const FuseA
 	auto kern = stencil3d_kernel<T, R, TYT, Fused>;
 	FI_LAUNCH(kern, grid, 32 * TYT, 0, s, g.size[0], g.size[1], g.size[2], zchunk, tab, p, q, fz, d_dot_out, d_partial, d_ticket,
 	          d_done);
+	note_stencil(FI_PCG_KERNEL_TILED_3D, R, false, TYT, chunks);
 }
 
 template <typename T>

@@ -438,6 +438,7 @@ void launch_ty(const Geom& g, const StencilTables& t, int chunks, const T* a, co
 	}
 	FI_LAUNCH(kern, grid, 256, smem, s, ma, mb, mc, g.size[0], g.size[1], g.nzl, g.zown0, g.zown1, g.zoff, g.size[2], zchunk, tab,
 	          static_cast<T>(t.gs2), q, p_new, st, par, d_dot_out, d_partial, d_ticket, d_done, epi);
+	note_stencil(FI_PCG_KERNEL_TMA_3D, R, GS, TY, chunks);
 }
 
 // Tile height.  Inside a long timed loop the GPU runs power-capped (SM clock ~1.78 of 1.97 GHz) and the kernel is bound by

@@ -31,7 +31,8 @@ extern "C" {
 /* 6: + fi_field_error_map (additions only) */
 /* 7: + fi_nearest_point_distance, fi_field_add_border_distance (additions only) */
 /* 8: + fi_field_mg_info, fi_field_mg_stage (additions only) */
-#define FI_B200_ABI_VERSION 8
+/* 9: + fi_field_pcg_stage (additions only) */
+#define FI_B200_ABI_VERSION 9
 
 #if defined(__GNUC__)
 #define FI_API __attribute__((visibility("default")))
@@ -459,6 +460,49 @@ enum {
  * vectors of the sizes above).  Runs the kernels the cycle runs, on scratch vectors of its own. */
 FI_API int fi_field_mg_stage(fi_field* f, const fi_solve_options* opt, int32_t stage, int32_t level, int64_t count, const float* in,
                              const float* in2, float* out);
+
+/* ---- Jacobi-PCG iteration, stage by stage (for tests) ---------------------------------------------------------- */
+/* One stage of the iteration fi_field_solve runs, on caller vectors and a caller scalar state, with the operator the
+ * solve builds for `opt` (precision FI_F32 or FI_F64, use_fast_stencil) and the same launch helpers, work buffers
+ * (r, q, the ring of directions, the parked step lengths, reduction scratch and tickets) and device-side flag. */
+#define FI_PCG_MAX_RING 8
+typedef struct fi_pcg_state {  /* PcgState of the solver plus the ring's parked step lengths */
+	double  rho[2];            /* r.M^-1 r by iteration parity: iteration k reads rho[k & 1] and writes rho[(k & 1) ^ 1] */
+	double  pq;                /* p.(S + P) p */
+	double  rr, bb, tol2bb, rr0;
+	int32_t done, breakdown;
+	int64_t iters, max_iters;
+	double  alpha[FI_PCG_MAX_RING - 1]; /* step lengths of the iterations whose x update is pending */
+} fi_pcg_state;
+
+enum {
+	FI_PCG_INIT    = 0, /* r = b - A x (vector X null: zero guess, A x not formed), dir[0] = M^-1 r; the whole state from b, r,
+	                     * opt->tolerance and opt->max_iterations (taken as given: no defaults substituted) */
+	FI_PCG_STENCIL = 1, /* fused direction+stencil step at ring position pos: p = dir[(pos + 1) % ring] = M^-1 r + beta dir[pos]
+	                     * (beta = 0 when iters == 0, else rho[par] / rho[par ^ 1]), q = S p, pq = p.q */
+	FI_PCG_DATA    = 2, /* q += P p, pq += p.P p with p = dir[(pos + 1) % ring] */
+	FI_PCG_UPDATE  = 3, /* update kernel of ring position pos (skip form; flush form at pos = ring - 1) */
+	FI_PCG_FLUSH   = 4, /* the flush after the loop: x += alpha[0] dir[1] + ... + alpha[count - 1] dir[count], 1 <= count < ring */
+	FI_PCG_UNFUSED = 5  /* the unfused iteration's pair without its operator application: x += a dir[0], r -= a q, rho, rr;
+	                     * then dir[0] = M^-1 r + beta dir[0] */
+};
+/* vectors[FI_PCG_V_*]: N elements each of the operator's precision, where `loc` says; vectors[FI_PCG_V_DIR + j] is dir[j],
+ * j < ring.  Every non-null vector is copied in before the stage and out after it; null ones enter as zeros (null B:
+ * the field's own A^T b). */
+enum { FI_PCG_V_X = 0, FI_PCG_V_R = 1, FI_PCG_V_Q = 2, FI_PCG_V_B = 3, FI_PCG_V_DIR = 4 };
+enum { FI_PCG_KERNEL_NONE = 0, FI_PCG_KERNEL_TMA_3D = 1, FI_PCG_KERNEL_TILED_3D = 2, FI_PCG_KERNEL_TMA_2D = 3 };
+enum { FI_PCG_DATA_CELLS = 1, FI_PCG_DATA_NODES = 2, FI_PCG_DATA_SPLIT = 4, FI_PCG_DATA_ROWS = 8 };
+typedef struct fi_pcg_report {  /* what the stage launched */
+	int32_t stencil;    /* FI_PCG_KERNEL_*: the fused stencil kernel (NONE: no fused kernel applies, nothing ran) */
+	int32_t radius;     /* R of its instantiation: 1, 2 or 4 */
+	int32_t gs;         /* 1: the gradient-smoothness instantiation */
+	int32_t tile_rows;  /* rows per tile (3D TMA: 7 or 8) */
+	int32_t z_chunks;   /* z chunks of the grid (3D) */
+	int32_t data_term;  /* FI_PCG_DATA_* mask of the data-term kernels launched */
+} fi_pcg_report;
+/* par: iteration parity (0 or 1); ring: 2, 4 or 8; count: FI_PCG_FLUSH only.  report is nullable. */
+FI_API int fi_field_pcg_stage(fi_field* f, const fi_solve_options* opt, int32_t stage, int32_t par, int32_t pos, int32_t ring, int32_t count,
+                              int32_t loc, void* const* vectors, fi_pcg_state* state, fi_pcg_report* report);
 
 #ifdef __cplusplus
 }
